@@ -34,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (no __pycache__ of tools/, oracle/)
 
 METRIC = "Mrays/s (primary+shadow+GI), 1080p 64-spp GI+DOF frame on LSVO 2048^3"
 UNIT = "Mrays/s"
@@ -277,12 +278,19 @@ def run_ours(args):
     sync_all()
     ev_start.record(stream)
     for i in range(args.steps):
-        fr.render_device(cam, w["spp"])
+        last = fr.render_device(cam, w["spp"])
     ev_end.record(stream)
     sync_all()
     kernel_times = ctx.take_kernel_timings()                 # ms of the dominant kernel (sort + trace) per frame, this rank
     ctx.set_option("time_frame_kernels", 0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed frame as the caller receives it (uint8 RGBA [H, W, 4]), stored as float32: 33 MB at 1080p; larger frames
+        # keep every k-th row so that the file, its .npy header (128 bytes) included, stays within 64 MB
+        img = last.cpu().numpy()
+        k = -(-img.size * 4 // (64_000_000 - 4096))
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "frame.npy"), img[::k].astype(np.float32))
     launches = ctx.launch_count - launches0
     ms_total = ev_start.elapsed_time(ev_end)
     kernel_ms = float(np.mean(kernel_times)) if kernel_times else float("nan")
@@ -445,7 +453,12 @@ def main():
     ap.add_argument("--split", default="tiles", choices=["tiles", "samples"])   # multi-GPU partition of the frame
     ap.add_argument("--no-extra", action="store_true")           # skip extra.one_bounce / extra.configs
     ap.add_argument("--cfg5-rays", type=int, default=100_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)   # writes DIR/frame.npy: the last timed frame
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the frame of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     # stdout must carry the ONE JSON line: libraries (NCCL's version banner, for one) printf to file descriptor 1, so the

@@ -61,7 +61,7 @@ def _f32(a):
 
 
 def build(quiet=True):
-    """(Re)build the checkers: the port always, oracle/_ref only where /root/reference exists."""
+    """(Re)build the checkers: the port always, oracle/_ref only where $VRT_REFERENCE names the reference tree."""
     subprocess.run(["make", "-s" if quiet else "-j1", "-C", HERE, "all"], check=True,
                    stdout=subprocess.DEVNULL if quiet else None)
 

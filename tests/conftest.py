@@ -61,7 +61,7 @@ def ref():
     from oracle import loader
     r = loader.ref()
     if r is None:
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
+        pytest.skip("oracle/_ref not built (needs the reference sources, see VRT_REFERENCE in oracle/Makefile)")
     return r
 
 
@@ -70,7 +70,7 @@ def ref_patched():
     from oracle import loader
     r = loader.ref_patched()
     if r is None:
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
+        pytest.skip("oracle/_ref not built (needs the reference sources, see VRT_REFERENCE in oracle/Makefile)")
     return r
 
 

@@ -1,5 +1,5 @@
-"""Generates the committed golden fixtures from the REFERENCE ITSELF (run in the container that has
-/root/reference and oracle/_ref built: `python tests/golden/make_golden.py`).
+"""Generates the committed golden fixtures from the REFERENCE ITSELF (needs a checkout of the reference's sources and
+oracle/_ref built from it: `VRT_REFERENCE=<checkout> make -C oracle && VRT_REFERENCE=<checkout> python tests/golden/make_golden.py`).
 
   textures.npz        res/grass_top_16x16.bmp, res/grass_side_16x16.bmp decoded to 16x16 RGB, top-down rows
                       (what sf::Image::loadFromFile presents; raycaster.hpp:53-54)
@@ -29,7 +29,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from oracle import loader  # noqa: E402
 
-REF = "/root/reference"
+REF = os.environ.get("VRT_REFERENCE", "")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -108,6 +108,7 @@ def make_cfg1_full(R):
 
 
 def main():
+    assert REF, "set VRT_REFERENCE to a checkout of the reference (johnBuffer/CpuVoxelRaycaster)"
     if len(sys.argv) > 1 and sys.argv[1] == "checker":
         make_checker_frames(loader.ref())
         return

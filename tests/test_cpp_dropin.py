@@ -78,13 +78,14 @@ def test_dropin_matches_python_api(vrt, ctx, terrain9_nodes, textures):
 
 
 # ---- the reference's own main loop against the drop-in headers ---------------------------------------------------------
-# The per-pixel path of /root/reference/src/main.cpp (lines 40-158: scene construction with FastNoise + SVO::setCell,
+# The per-pixel path of the reference's src/main.cpp (lines 40-158: scene construction with FastNoise + SVO::setCell,
 # LSVO(const SVO&), Camera, RayCaster, the autofocus rule, the swarm lambda with Camera::getRay + RayCaster::renderRay,
 # samples_to_image) is compiled UNCHANGED against include/vrt/compat.hpp.  Only what the judge of a drop-in would change is
 # changed, by the rules below: the #include block, and the lines that talk to the SFML window / input / presentation.
-# The source is generated into a temporary directory from the reference tree where it lies (never copied into the repo);
-# the binary is built where /root/reference exists and travels to the GPU box with the snapshot.
-REF_MAIN = "/root/reference/src/main.cpp"
+# The source is generated into a temporary directory from the reference tree where it lies (never copied into the repo): a
+# checkout of johnBuffer/CpuVoxelRaycaster named by the environment variable VRT_REFERENCE.  Without one both tests skip.
+REF = os.environ.get("VRT_REFERENCE")
+REF_MAIN = os.path.join(REF, "src", "main.cpp") if REF else None
 MAIN_EXE = os.path.join(ROOT, "tests", "cpp", "main_dropin")
 
 
@@ -155,8 +156,8 @@ def write_bmp24(path, rgb):
 
 
 def test_reference_main_loop_compiles_against_the_dropin_headers(vrt):
-    if not os.path.exists(REF_MAIN):
-        pytest.skip("/root/reference absent: the binary built in the container is used")
+    if not (REF_MAIN and os.path.exists(REF_MAIN)):
+        pytest.skip("needs the reference's src/main.cpp (VRT_REFERENCE)")
     src = build_main_dropin()
     # the hot-path lines are the reference's own, untouched
     for needle in ("volume_raw->setCell(Cell::Solid, Cell::Grass, x, y + 256, z);", "LSVO<max_depth> lsvo(*volume_raw);",
@@ -176,10 +177,10 @@ def test_reference_main_loop_runs_on_the_gpu(vrt, ctx, terrain9_nodes, textures,
     """The generated main() — the reference's loop, per-pixel Camera::getRay + RayCaster::renderRay calls queued and shaded in
     one launch per frame — renders the demo's 960x540 checkerboard frames; the image equals the batched RayCaster.render()
     path (Python mirror) byte for byte, with and without the GI pass."""
-    if os.path.exists(REF_MAIN):
+    if REF_MAIN and os.path.exists(REF_MAIN):
         build_main_dropin()
     if not os.path.exists(MAIN_EXE):
-        pytest.skip("tests/cpp/main_dropin was not built (needs /root/reference)")
+        pytest.skip("tests/cpp/main_dropin was not built (needs the reference's src/main.cpp, VRT_REFERENCE)")
     (tmp_path / "res").mkdir()
     write_bmp24(str(tmp_path / "res" / "grass_top_16x16.bmp"), textures[0])
     write_bmp24(str(tmp_path / "res" / "grass_side_16x16.bmp"), textures[1])

@@ -1,5 +1,5 @@
 """Pins the CPU restatement (oracle/port.c) against the reference's OWN compiled sources (oracle/_ref, built by
-oracle/Makefile from /root/reference).  Skipped where oracle/_ref has not been built.  Bit-exact, except the
+oracle/Makefile from the checkout $VRT_REFERENCE names).  Skipped where oracle/_ref has not been built.  Bit-exact, except the
 stochastic frame, which the reference cannot reproduce even against itself (racy global RNG): PSNR there."""
 import numpy as np
 import pytest
