@@ -996,6 +996,10 @@ static void grid_render_range(void* c_, uint64_t b, uint64_t e) {
     for (uint64_t i = b; i < e; ++i) {
         const int32_t y = p->row_begin + (int32_t)(i / W), x = (int32_t)(i % W);
         if (p->tile_step > 1 && (((y - p->row_begin) >> 2) % p->tile_step) != p->tile_index) continue;
+        if (p->checker) {                                                                           /* main.cpp:143, as vo_render */
+            const int32_t rel = p->checker_area_height > 0 ? y % p->checker_area_height : y;
+            if ((rel & 1) != ((x + p->checker - 1) & 1)) continue;
+        }
         const size_t px = (size_t)y * W + (size_t)x;
         uint32_t* a = c->accum + 4 * px;
         for (int32_t s = 0; s < p->spp; ++s) {

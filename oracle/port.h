@@ -120,7 +120,8 @@ void vo_render(const vo_lnode* nodes, const vo_render_params* p, const uint8_t* 
  *   otherwise (Solid, or Mirror at max depth): albedo = texture (top iff n.y != 0; texel index min(15, uint(16*uv))),
  *     shadow ray o = hit + n * 0.001 toward the light, light = unoccluded ? max(0, dot(to_light, n)) : 0,
  *     colour = mult(mult(albedo, clamp01(light)), tint) (utils.cpp:43-48).
- * cells[(x*Y+y)*Z+z] = Cell::Type.  stats->rays: [0] primary, [1] shadow, [2] reflection rays. */
+ * cells[(x*Y+y)*Z+z] = Cell::Type.  stats->rays: [0] primary, [1] shadow, [2] reflection rays.
+ * checker / checker_area_height select pixels as in vo_render; the other pixels of accum and rgba are left alone. */
 void vo_grid_render(const uint8_t* cells, int X, int Y, int Z, const vo_render_params* p, const uint8_t* tex_top,
                     const uint8_t* tex_side, uint32_t* accum, uint8_t* rgba, vo_render_stats* stats);
 

@@ -8,21 +8,28 @@ import pytest
 
 from conftest import ROOT, golden
 
-EXE = os.path.join(ROOT, "tests", "cpp", "dropin_test")
-TEX = os.path.join(ROOT, "tests", "cpp", "textures.bin")
 
 
-def build():
+@pytest.fixture(scope="module")
+def bin_dir(tmp_path_factory):
+    """The test programs and their inputs are written outside the source tree, which may be read-only."""
+    return str(tmp_path_factory.mktemp("cpp"))
+
+
+def build(bin_dir):
+    exe, tex = os.path.join(bin_dir, "dropin_test"), os.path.join(bin_dir, "textures.bin")
     lib_dir = os.path.join(ROOT, "cpuvoxelraycaster_b200")
     subprocess.run(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-I" + os.path.join(ROOT, "include"),
-                    os.path.join(ROOT, "tests", "cpp", "dropin_test.cpp"), "-o", EXE, "-L" + lib_dir, "-lvrt",
+                    os.path.join(ROOT, "tests", "cpp", "dropin_test.cpp"), "-o", exe, "-L" + lib_dir, "-lvrt",
                     "-Wl,-rpath," + lib_dir], check=True)
     t = golden("textures.npz")
-    open(TEX, "wb").write(t["top"].tobytes() + t["side"].tobytes())
+    with open(tex, "wb") as f:
+        f.write(t["top"].tobytes() + t["side"].tobytes())
+    return exe, tex
 
 
-def test_dropin_compiles_and_fails_loudly_without_gpu(vrt):
-    build()
+def test_dropin_compiles_and_fails_loudly_without_gpu(vrt, bin_dir):
+    EXE, TEX = build(bin_dir)
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present: covered by the gpu test")
@@ -31,8 +38,8 @@ def test_dropin_compiles_and_fails_loudly_without_gpu(vrt):
 
 
 @pytest.mark.gpu
-def test_dropin_matches_python_api(vrt, ctx, terrain9_nodes, textures):
-    build()
+def test_dropin_matches_python_api(vrt, ctx, terrain9_nodes, textures, bin_dir):
+    EXE, TEX = build(bin_dir)
     r = subprocess.run([EXE, TEX], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout + r.stderr
     out = {}
@@ -86,7 +93,6 @@ def test_dropin_matches_python_api(vrt, ctx, terrain9_nodes, textures):
 # checkout of johnBuffer/CpuVoxelRaycaster named by the environment variable VRT_REFERENCE.  Without one both tests skip.
 REF = os.environ.get("VRT_REFERENCE")
 REF_MAIN = os.path.join(REF, "src", "main.cpp") if REF else None
-MAIN_EXE = os.path.join(ROOT, "tests", "cpp", "main_dropin")
 
 
 def generate_main_dropin(text):
@@ -133,18 +139,18 @@ def generate_main_dropin(text):
     return src
 
 
-def build_main_dropin():
-    import tempfile
+def build_main_dropin(bin_dir):
+    """Returns (generated source, path of the program built from it in bin_dir)."""
     text = open(REF_MAIN).read()
     src = generate_main_dropin(text)
     lib_dir = os.path.join(ROOT, "cpuvoxelraycaster_b200")
-    with tempfile.TemporaryDirectory() as d:
-        path = os.path.join(d, "main_dropin.cpp")
-        open(path, "w").write(src)
-        r = subprocess.run(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-I" + os.path.join(ROOT, "include"), path, "-o", MAIN_EXE,
-                            "-L" + lib_dir, "-lvrt", "-Wl,-rpath," + lib_dir], capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr[-4000:] + "\n----\n" + "\n".join("%4d %s" % (n + 1, l) for n, l in enumerate(src.splitlines()))
-    return src
+    path, exe = os.path.join(bin_dir, "main_dropin.cpp"), os.path.join(bin_dir, "main_dropin")
+    with open(path, "w") as f:
+        f.write(src)
+    r = subprocess.run(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-I" + os.path.join(ROOT, "include"), path, "-o", exe,
+                        "-L" + lib_dir, "-lvrt", "-Wl,-rpath," + lib_dir], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-4000:] + "\n----\n" + "\n".join("%4d %s" % (n + 1, l) for n, l in enumerate(src.splitlines()))
+    return src, exe
 
 
 def write_bmp24(path, rgb):
@@ -155,10 +161,10 @@ def write_bmp24(path, rgb):
     open(path, "wb").write(b"BM" + struct.pack("<IHHI", 54 + len(rows), 0, 0, 54) + struct.pack("<IiiHHIIiiII", 40, w, h, 1, 24, 0, len(rows), 2835, 2835, 0, 0) + rows)
 
 
-def test_reference_main_loop_compiles_against_the_dropin_headers(vrt):
+def test_reference_main_loop_compiles_against_the_dropin_headers(vrt, bin_dir):
     if not (REF_MAIN and os.path.exists(REF_MAIN)):
         pytest.skip("needs the reference's src/main.cpp (VRT_REFERENCE)")
-    src = build_main_dropin()
+    src, MAIN_EXE = build_main_dropin(bin_dir)
     # the hot-path lines are the reference's own, untouched
     for needle in ("volume_raw->setCell(Cell::Solid, Cell::Grass, x, y + 256, z);", "LSVO<max_depth> lsvo(*volume_raw);",
                    "HitPoint closest_point = camera.getClosestPoint(lsvo);", "const CameraRay camera_ray = camera.getRay(glm::vec2(lens_x, lens_y));",
@@ -167,20 +173,19 @@ def test_reference_main_loop_compiles_against_the_dropin_headers(vrt):
         assert needle in src, needle
     import torch
     if not torch.cuda.is_available():
-        r = subprocess.run([MAIN_EXE, "1"], capture_output=True, text=True, cwd=os.path.join(ROOT, "tests", "cpp"))
+        r = subprocess.run([MAIN_EXE, "1"], capture_output=True, text=True, cwd=bin_dir)
         assert r.returncode != 0 and "libvrt error -2" in (r.stdout + r.stderr)      # fails loudly without a device
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("use_gi", [0, 1])
-def test_reference_main_loop_runs_on_the_gpu(vrt, ctx, terrain9_nodes, textures, use_gi, tmp_path):
+def test_reference_main_loop_runs_on_the_gpu(vrt, ctx, terrain9_nodes, textures, use_gi, tmp_path, bin_dir):
     """The generated main() — the reference's loop, per-pixel Camera::getRay + RayCaster::renderRay calls queued and shaded in
     one launch per frame — renders the demo's 960x540 checkerboard frames; the image equals the batched RayCaster.render()
     path (Python mirror) byte for byte, with and without the GI pass."""
-    if REF_MAIN and os.path.exists(REF_MAIN):
-        build_main_dropin()
-    if not os.path.exists(MAIN_EXE):
-        pytest.skip("tests/cpp/main_dropin was not built (needs the reference's src/main.cpp, VRT_REFERENCE)")
+    if not (REF_MAIN and os.path.exists(REF_MAIN)):
+        pytest.skip("needs the reference's src/main.cpp (VRT_REFERENCE)")
+    _, MAIN_EXE = build_main_dropin(bin_dir)
     (tmp_path / "res").mkdir()
     write_bmp24(str(tmp_path / "res" / "grass_top_16x16.bmp"), textures[0])
     write_bmp24(str(tmp_path / "res" / "grass_side_16x16.bmp"), textures[1])

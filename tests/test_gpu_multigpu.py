@@ -23,19 +23,20 @@ def test_frame_identical_across_world_sizes():
 
 
 @pytest.mark.gpu
-def test_cpp_host_drives_several_gpus_through_the_c_abi():
+def test_cpp_host_drives_several_gpus_through_the_c_abi(tmp_path):
     """tests/cpp/multigpu_test.cpp: one C++ process, vrt_comm_create_local + vrt_render_distributed on 2-4 GPUs, tile and sample
     splits, three pipelined frames each, compared byte for byte with vrt_render on one GPU."""
     import torch
     from conftest import golden
     if torch.cuda.device_count() < 2:
         pytest.skip("one GPU visible")
-    exe, tex = os.path.join(ROOT, "tests", "cpp", "multigpu_test"), os.path.join(ROOT, "tests", "cpp", "textures.bin")
+    exe, tex = str(tmp_path / "multigpu_test"), str(tmp_path / "textures.bin")          # outside the (possibly read-only) source tree
     lib_dir = os.path.join(ROOT, "cpuvoxelraycaster_b200")
     subprocess.run(["g++", "-O2", "-std=c++17", "-I" + os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "cpp", "multigpu_test.cpp"),
                     "-o", exe, "-L" + lib_dir, "-lvrt", "-Wl,-rpath," + lib_dir], check=True)
     t = golden("textures.npz")
-    open(tex, "wb").write(t["top"].tobytes() + t["side"].tobytes())
+    with open(tex, "wb") as fh:
+        fh.write(t["top"].tobytes() + t["side"].tobytes())
     # three or more GPUs when the box has them: that is where an arrival protocol can go wrong (a fast rank overtaking a slow one)
     r = subprocess.run([exe, tex, str(min(4, torch.cuda.device_count()))], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "multigpu_test: OK" in r.stdout and "MISMATCH" not in r.stdout, r.stdout[-3000:] + r.stderr[-2000:]

@@ -231,3 +231,38 @@ def test_checkerboard_frames(port, vrt, textures):
             p.checker = 1 + (frame & 1)
             acc += port.render(nodes, p, *textures)[0]
         assert np.array_equal(acc, g["samples2_" + tag]), tag
+
+
+def test_grid_render_checkerboard_halves(port):
+    """vo_grid_render with the checkerboard of main.cpp:143 (the rule vo_render applies): it touches exactly the pixels the rule
+    selects, those pixels equal the full frame's, the others are left alone, and the two halves add up to the full frame."""
+    h = port.terrain_heights(64)
+    y = np.arange(64)[None, :, None]
+    cells = (y <= (20 + np.clip(h, 0, 30))[:, None, :]).astype(np.uint8)
+    xs, zs = np.nonzero(h <= 12)
+    cells[xs, 20 + np.clip(h, 0, 30)[xs, zs], zs] = 2               # a mirror lake on the lowest columns
+    from oracle import loader
+    W, H = 53, 31
+    p = loader.PortRenderParams()
+    p.width, p.height, p.depth, p.guard = W, H, 6, 6
+    p.cam_position[:] = [32.0, 60.0, 4.0]
+    p.rot_mat[:] = [1.0, 0.0, 0.0, 0.0, 0.6, -0.8, 0.0, 0.8, 0.6]                 # looking down towards +z
+    p.fov, p.aperture, p.focal_length = 1.0, 0.3, 30.0
+    p.light_position[:] = [100.0, 300.0, -50.0]
+    p.use_gi, p.gi_bounces, p.use_samples, p.spp = 0, 1, 1, 2
+    p.seed_lo, p.threads, p.roughness, p.max_bounds = 0x5EED, 4, 0.1, 4
+    full, full_rgba, _ = port.grid_render(cells, p, np.full(768, 200, np.uint8), np.full(768, 120, np.uint8))
+    assert (full[..., 3] == 2).all() and full_rgba[..., :3].max() > 0
+    xs, ys = np.meshgrid(np.arange(W), np.arange(H))
+    for area in (0, 7):
+        rel = ys % area if area else ys
+        halves = np.zeros_like(full)
+        for checker in (1, 2):
+            p.checker, p.checker_area_height = checker, area
+            accum, rgba, _ = port.grid_render(cells, p, np.full(768, 200, np.uint8), np.full(768, 120, np.uint8))
+            rule = (rel & 1) == ((xs + checker - 1) & 1)
+            assert np.array_equal(accum[..., 3] > 0, rule), (area, checker)
+            assert np.array_equal(accum[rule], full[rule]) and np.array_equal(rgba[rule], full_rgba[rule])
+            assert not accum[~rule].any() and not rgba[~rule].any()
+            halves += accum
+        assert np.array_equal(halves, full)
