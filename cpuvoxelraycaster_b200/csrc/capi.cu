@@ -675,6 +675,9 @@ int check_render_args(const vrt_scene* sc, const vrt_camera* cam, const vrt_rend
     if (p->width <= 0 || p->height <= 0 || p->width > 65536 || p->height > 65536) return fail(VRT_ERR_INVALID, std::string(who) + ": bad frame size");
     if (p->row_begin < 0 || p->row_end > p->height || p->row_begin > p->row_end) return fail(VRT_ERR_INVALID, std::string(who) + ": bad row range");
     if (cam && (p->spp <= 0 || p->gi_bounces < 0 || p->gi_bounces > 2)) return fail(VRT_ERR_INVALID, std::string(who) + ": spp must be > 0 and gi_bounces in 0..2");
+    // the resolve blends the accumulated colour as ONE 8-bit sample: spp sums would wrap around
+    if (cam && !p->use_samples && p->spp != 1)
+        return fail(VRT_ERR_INVALID, std::string(who) + ": the temporal-blend mode renders one sample per frame (raycaster.hpp:77-85)");
     if (p->tile_step > 1 && (p->tile_index < 0 || p->tile_index >= p->tile_step)) return fail(VRT_ERR_INVALID, std::string(who) + ": tile_index must be in [0, tile_step)");
     if (cam && !sc->has_tex) return fail(VRT_ERR_INVALID, std::string(who) + ": call vrt_scene_set_textures first (raycaster.hpp:53-54)");
     if (cam)    // a rotation (camera_controller.hpp:27-32): the frame kernels rely on |ray direction| staying near 1 (Trav2, kUnit)
@@ -883,7 +886,6 @@ int vrt_render(vrt_scene* sc, const vrt_camera* cam, const vrt_render_params* p,
                vrt_render_stats* stats) {
     if (!cam || !rgba) return fail(VRT_ERR_INVALID, "vrt_render: NULL argument");
     if (int s = check_render_args(sc, cam, p, "vrt_render")) return s;
-    if (!p->use_samples && p->spp != 1) return fail(VRT_ERR_INVALID, "vrt_render: the temporal-blend mode renders one sample per frame (raycaster.hpp:77-85)");
     vrt_context* ctx = sc->ctx;
     if (int s = use_device(ctx)) return s;
     const size_t px = size_t(p->width) * p->height;

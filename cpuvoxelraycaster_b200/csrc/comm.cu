@@ -176,6 +176,20 @@ __global__ void __launch_bounds__(256) resolve_push_kernel(Sources src, Targets 
     for (int t = 0; t < dst.n; ++t) reinterpret_cast<uchar4*>(dst.frame[t])[i] = out;   // peer store over NVLink
 }
 
+// Loads the communicator's kernels into the current context.  With lazy module loading (the CUDA 12 default) a kernel is loaded
+// at its first launch, and loading may synchronise the context: a first launch queued behind a spin kernel then blocks the host
+// until the spin ends — which, with one thread driving several ranks, waits for ranks that thread has not enqueued yet (seen on
+// one GPU: the first sample-split frame timed out in resolve_push_kernel<true>).
+cudaError_t load_comm_kernels() {
+    const void* kernels[] = {reinterpret_cast<const void*>(signal_kernel), reinterpret_cast<const void*>(set_kernel),
+                             reinterpret_cast<const void*>(wait_all_kernel), reinterpret_cast<const void*>(wait_kernel),
+                             reinterpret_cast<const void*>(resolve_push_kernel<false>), reinterpret_cast<const void*>(resolve_push_kernel<true>)};
+    cudaFuncAttributes a;
+    for (const void* k : kernels)
+        if (cudaError_t e = cudaFuncGetAttributes(&a, k)) return e;
+    return cudaSuccess;
+}
+
 int check_comm(const vrt_comm* c, const char* who) {
     if (!c) return fail(VRT_ERR_INVALID, std::string(who) + ": comm is NULL");
     if (!c->connected) return fail(VRT_ERR_INVALID, std::string(who) + ": call vrt_comm_connect first");
@@ -187,6 +201,7 @@ int comm_alloc(vrt_context* ctx, int rank, int world, int width, int height, vrt
     if (world < 1 || world > kMaxWorld || rank < 0 || rank >= world) return fail(VRT_ERR_INVALID, std::string(who) + ": need 0 <= rank < world <= 16");
     if (width <= 0 || height <= 0 || width > 65536 || height > 65536) return fail(VRT_ERR_INVALID, std::string(who) + ": bad frame size");
     if (int s = use_device(ctx)) return s;
+    if (cudaError_t e = load_comm_kernels()) return cuda_fail(e, who);
     vrt_comm* c = new (std::nothrow) vrt_comm();
     if (!c) return fail(VRT_ERR_OOM, std::string(who) + ": host allocation failed");
     c->ctx = ctx; c->rank = rank; c->world = world; c->width = width; c->height = height;
@@ -332,8 +347,9 @@ int vrt_render_distributed(vrt_comm* c, vrt_scene* sc, const vrt_camera* cam, co
     uint32_t* accum = c->accum(c->rank);
     Flags* rf = c->flags(root);
 
-    // sample split: the peers read this accumulator during their reduce of the previous frame — wait for all of them
-    if (split == VRT_SPLIT_SAMPLES && W > 1 && c->sample_frames > 0) {
+    // the peers read this accumulator during their reduce of the latest sample-split frame — wait for all of them before it is
+    // cleared, whichever split this frame uses
+    if (W > 1 && c->sample_frames > 0) {
         wait_kernel<<<1, 1, 0, st>>>(&rf->reduced, c->sample_frames * uint64_t(W), &c->flags(c->rank)->error);
         ctx->launches += 1;
     }

@@ -223,8 +223,8 @@ class FrameRenderer:
 
     def render_pipelined(self, camera, spp, sample_offset=0):
         """Streaming form of render() for the peer exchange: enqueues this frame (its host copy runs on a second stream
-        while the next frame renders) and returns the PREVIOUS frame's host image (None for the first call); call
-        flush() after the last frame.  K calls + flush() deliver K frames."""
+        while the next frame renders) and returns None.  K calls + flush() deliver K frames: frame i (counted by
+        frames_done) is copied to host_frames[i & 1], so after flush() the last two frames are in host memory."""
         assert self.peer is not None, "render_pipelined needs the peer exchange"
         p = self.params(spp, sample_offset)
         i = self.frames_done

@@ -222,7 +222,7 @@ typedef struct vrt_render_params {
     float light_position[3];     /* RayCaster::light_position (normalised, main.cpp:126) */
     int32_t use_gi;              /* RayCaster::use_gi */
     int32_t gi_bounces;          /* 1 = reference; 2 = extension (DESIGN.md) */
-    int32_t use_samples;         /* RayCaster::use_samples */
+    int32_t use_samples;         /* RayCaster::use_samples; 0 = the temporal blend, one sample per frame (spp must be 1) */
     int32_t accum_in;            /* vrt_render: 1 = `accum` holds earlier sums and is added to (progressive frames) */
     int32_t tile_step;           /* > 1: only 4-row tiles t (counted from row_begin) with t % tile_step == tile_index */
     int32_t tile_index;          /*      are rendered/resolved — the balanced multi-GPU row partition */
@@ -335,7 +335,8 @@ int vrt_autofocus(vrt_scene* scene, const vrt_camera* cam, float* focal_length);
  * host_rgba is given on a receiving rank, copied to it on a second stream while the next frame renders.
  * vrt_render_distributed only enqueues; vrt_comm_frame_wait blocks until the last frame (and its host copy) is complete
  * and reports a peer that failed to show up.  Every member must call vrt_render_distributed for every frame with the
- * same camera, parameters and split; row_begin/row_end/tile_step/tile_index/sample_offset/accum_in of *p are ignored. */
+ * same camera, parameters and split; row_begin/row_end/tile_step/tile_index/accum_in of *p are ignored, sample_offset is
+ * the index of the frame's first sample as in vrt_render. */
 typedef struct vrt_comm vrt_comm;
 #define VRT_COMM_HANDLE_BYTES 256
 typedef enum vrt_split { VRT_SPLIT_TILES = 0, VRT_SPLIT_SAMPLES = 1 } vrt_split;

@@ -2,13 +2,16 @@
 // main.cpp with RayCaster::render in place of the swarm lambda of src/main.cpp:139-154 — does to use a whole box.
 // Builds the demo terrain T(9) on every GPU, renders GI + DOF frames with the frame split over the GPUs by tiles and by
 // samples (vrt_comm_create_local + vrt_render_distributed) and compares every delivered frame byte for byte with the
-// same frame rendered on GPU 0 alone (vrt_render).  usage: multigpu_test <textures.bin> [n_gpus]
+// same frame rendered on GPU 0 alone (vrt_render).  usage: multigpu_test <textures.bin> [n_gpus] [one_device]
+// one_device = 1: every rank is a context on device 0 with its own stream — the whole protocol (arrival counters, the
+// sample-split reduce, deliver_all, the double-buffer waits) then runs on a single GPU.
 // exit code 0 = identical, 3 = fewer than 2 CUDA devices (nothing to test), 1 = mismatch / error.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <vector>
 
+#include <cuda_runtime.h>
 #include <vrt.h>
 
 #define CHECK(call)                                                                          \
@@ -27,11 +30,12 @@ int main(int argc, char** argv) {
     if (!f || std::fread(tex.data(), 1, 1536, f) != 1536) { std::fprintf(stderr, "cannot read textures\n"); return 2; }
     std::fclose(f);
     const int want = argc > 2 ? std::atoi(argv[2]) : 2;
+    const bool one_device = argc > 3 && std::atoi(argv[3]) != 0;
 
     std::vector<vrt_context*> ctx;
     for (int d = 0; d < want; ++d) {
         vrt_context* c = nullptr;
-        const int s = vrt_context_create(d, nullptr, &c);
+        const int s = vrt_context_create(one_device ? 0 : d, nullptr, &c);       // a non-blocking stream of its own
         if (s != VRT_OK) break;
         ctx.push_back(c);
     }
@@ -84,12 +88,28 @@ int main(int argc, char** argv) {
             bad += !same;
         }
     }
-    // deliver_all: every GPU receives the frame in its own memory
+    // deliver_all: every GPU receives the frame in its own memory and copies it to its own host buffer.  The buffers are pinned:
+    // a copy into pageable memory returns only once it is done, so the first rank's call would wait for ranks not yet enqueued.
     {
         vrt_render_params q = p;
         q.sample_offset = 0;
-        for (int r = 0; r < world; ++r) CHECK(vrt_render_distributed(comm[r], scene[r], &cam, &q, VRT_SPLIT_TILES, 1, nullptr));
+        const size_t bytes = size_t(W) * H * 4;
+        std::vector<uint8_t*> host(world, nullptr);
+        for (int r = 0; r < world; ++r) {
+            if (cudaHostAlloc(reinterpret_cast<void**>(&host[r]), bytes, cudaHostAllocPortable) != cudaSuccess) {
+                std::printf("cudaHostAlloc failed\n");
+                return 1;
+            }
+            std::memset(host[r], 0x5A, bytes);
+        }
+        for (int r = 0; r < world; ++r) CHECK(vrt_render_distributed(comm[r], scene[r], &cam, &q, VRT_SPLIT_TILES, 1, host[r]));
         for (int r = 0; r < world; ++r) CHECK(vrt_comm_frame_wait(comm[r]));
+        for (int r = 0; r < world; ++r) {
+            const bool same = std::memcmp(host[r], single[0].data(), bytes) == 0;
+            std::printf("world=%d deliver_all rank=%d: %s\n", world, r, same ? "identical" : "MISMATCH");
+            bad += !same;
+            cudaFreeHost(host[r]);
+        }
         uint64_t frames = 0;
         CHECK(vrt_comm_info(comm[world - 1], nullptr, nullptr, &frames));
         uint8_t* d = nullptr;
