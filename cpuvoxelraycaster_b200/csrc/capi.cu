@@ -473,6 +473,19 @@ int vrt_scene_set_cells(vrt_scene* sc, const uint32_t* xyz, uint64_t n, int32_t 
     ctx->launches += 3;
     if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? fail(VRT_ERR_OOM, "vrt_scene_set_cells: device allocation failed")
                                                                 : cuda_fail(e, "vrt_scene_set_cells");
+    // a painted scene: surviving voxels keep their colour, added ones get 1
+    const bool painted = sc->voxel_colors.ptr != nullptr;
+    if (painted) {
+        e = sc->voxel_colors_next.reserve(size_t(n_merged) + n_merged / 16 + 4096);    // slack: edits change the count a little
+        if (e == cudaSuccess)
+            e = vrt::launch_gather_key_colors(sc->d_voxel_keys, static_cast<const uint8_t*>(sc->voxel_colors.ptr), sc->n_voxel_keys, d_merged,
+                                              n_merged, static_cast<uint8_t*>(sc->voxel_colors_next.ptr), ctx->stream);
+        ctx->launches += 1;
+        if (e != cudaSuccess) {
+            cudaFree(d_merged);
+            return e == cudaErrorMemoryAllocation ? fail(VRT_ERR_OOM, "vrt_scene_set_cells: device allocation failed") : cuda_fail(e, "vrt_scene_set_cells");
+        }
+    }
     // staged: the node array is rebuilt from the candidate key set first; the resident keys are replaced only when that worked
     if (int s = rebuild_from_keys(sc, d_merged, n_merged, "vrt_scene_set_cells", true)) {
         cudaFree(d_merged);
@@ -481,8 +494,89 @@ int vrt_scene_set_cells(vrt_scene* sc, const uint32_t* xyz, uint64_t n, int32_t 
     cudaFree(sc->d_voxel_keys);
     sc->device_bytes += uint64_t(n_merged) * sizeof(uint64_t);
     sc->device_bytes -= uint64_t(sc->n_voxel_keys) * sizeof(uint64_t);
+    if (painted) {
+        std::swap(sc->voxel_colors, sc->voxel_colors_next);
+        sc->device_bytes += n_merged;
+        sc->device_bytes -= sc->n_voxel_keys;
+    }
     sc->d_voxel_keys = d_merged;
     sc->n_voxel_keys = n_merged;
+    if (painted) {                                          // the new leaf slots carry LNode()'s colour 1 until stamped
+        VRT_CUDA(vrt::launch_stamp_key_colors(sc->d_nodes, int(sc->depth), sc->d_voxel_keys, static_cast<const uint8_t*>(sc->voxel_colors.ptr),
+                                              sc->n_voxel_keys, ctx->stream));
+        ctx->launches += 1;
+        VRT_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return VRT_OK;
+}
+
+namespace {
+// checks a voxel list (setCell coordinates) and copies it into a device buffer with `tail_bytes` more behind it, filled from
+// `tail` unless that is NULL (caller frees)
+int upload_cells(vrt_scene* sc, const uint32_t* xyz, uint64_t n, const void* tail, size_t tail_bytes, uint32_t** d_xyz, const char* who) {
+    *d_xyz = nullptr;
+    if (n > 0x7fffffffull) return fail(VRT_ERR_INVALID, std::string(who) + ": too many voxels");
+    const uint32_t S = 1u << sc->depth;
+    for (uint64_t i = 0; i < 3 * n; ++i)
+        if (xyz[i] >= S) return fail(VRT_ERR_INVALID, std::string(who) + ": voxel out of range (UB in the reference, svo.hpp:72)");
+    if (int s = use_device(sc->ctx)) return s;
+    const size_t bytes = size_t(n) * 3 * sizeof(uint32_t);
+    cudaError_t e = cudaMalloc(d_xyz, bytes + tail_bytes);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(*d_xyz, xyz, bytes, cudaMemcpyHostToDevice, sc->ctx->stream);
+    if (e == cudaSuccess && tail) e = cudaMemcpyAsync(reinterpret_cast<char*>(*d_xyz) + bytes, tail, tail_bytes, cudaMemcpyHostToDevice, sc->ctx->stream);
+    if (e != cudaSuccess) {
+        if (*d_xyz) cudaFree(*d_xyz);
+        *d_xyz = nullptr;
+        return e == cudaErrorMemoryAllocation ? fail(VRT_ERR_OOM, std::string(who) + ": device allocation failed") : cuda_fail(e, who);
+    }
+    return VRT_OK;
+}
+}  // namespace
+
+int vrt_scene_paint_cells(vrt_scene* sc, const uint32_t* xyz, const uint8_t* colors, uint64_t n, uint64_t* painted) {
+    if (!sc) return fail(VRT_ERR_INVALID, "vrt_scene_paint_cells: scene is NULL");
+    if (sc->kind != VRT_SCENE_LSVO || sc->d_heights)
+        return fail(VRT_ERR_UNSUPPORTED, "vrt_scene_paint_cells: needs an LSVO scene that is not a heightfield (every height edit re-flattens it)");
+    if (n && (!xyz || !colors)) return fail(VRT_ERR_INVALID, "vrt_scene_paint_cells: NULL voxel or colour list");
+    if (painted) *painted = 0;
+    if (n == 0) return VRT_OK;
+    uint32_t* d_xyz = nullptr;
+    if (int s = upload_cells(sc, xyz, n, colors, size_t(n), &d_xyz, "vrt_scene_paint_cells")) return s;
+    vrt_context* ctx = sc->ctx;
+    cudaError_t e = cudaSuccess;
+    if (sc->d_voxel_keys && !sc->voxel_colors.ptr) {         // first paint of a voxel-set scene: every voxel has LNode()'s colour 1
+        e = sc->voxel_colors.reserve(size_t(sc->n_voxel_keys) + sc->n_voxel_keys / 16 + 4096);
+        if (e == cudaSuccess) e = cudaMemsetAsync(sc->voxel_colors.ptr, 1, sc->n_voxel_keys, ctx->stream);
+        if (e == cudaSuccess) sc->device_bytes += sc->n_voxel_keys;
+        else sc->voxel_colors.release();
+    }
+    uint64_t count = 0;
+    if (e == cudaSuccess)
+        e = vrt::device_paint_cells(sc->d_nodes, int(sc->depth), d_xyz, reinterpret_cast<const uint8_t*>(d_xyz + 3 * n), n, sc->d_voxel_keys,
+                                    sc->n_voxel_keys, static_cast<uint8_t*>(sc->voxel_colors.ptr), &count, ctx->stream);
+    ctx->launches += 3;                                       // leaf slots, sort, write
+    cudaFree(d_xyz);
+    if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? fail(VRT_ERR_OOM, "vrt_scene_paint_cells: device allocation failed")
+                                                                : cuda_fail(e, "vrt_scene_paint_cells");
+    if (painted) *painted = count;
+    return VRT_OK;
+}
+
+int vrt_scene_cell_colors(vrt_scene* sc, const uint32_t* xyz, uint64_t n, int16_t* out) {
+    if (!sc) return fail(VRT_ERR_INVALID, "vrt_scene_cell_colors: scene is NULL");
+    if (sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, "vrt_scene_cell_colors: needs an LSVO scene");
+    if (n && (!xyz || !out)) return fail(VRT_ERR_INVALID, "vrt_scene_cell_colors: NULL buffer");
+    if (n == 0) return VRT_OK;
+    uint32_t* d_xyz = nullptr;
+    if (int s = upload_cells(sc, xyz, n, nullptr, size_t(n) * sizeof(int16_t), &d_xyz, "vrt_scene_cell_colors")) return s;
+    vrt_context* ctx = sc->ctx;
+    int16_t* d_out = reinterpret_cast<int16_t*>(d_xyz + 3 * n);
+    cudaError_t e = vrt::launch_cell_colors(sc->d_nodes, int(sc->depth), d_xyz, n, d_out, ctx->stream);
+    ctx->launches += 1;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, size_t(n) * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    cudaFree(d_xyz);
+    if (e != cudaSuccess) return cuda_fail(e, "vrt_scene_cell_colors");
     return VRT_OK;
 }
 
@@ -570,6 +664,8 @@ int vrt_scene_destroy(vrt_scene* sc) {
     sc->beam_floor.release();
     sc->build_pool.release();
     sc->edit_old.release();
+    sc->voxel_colors.release();
+    sc->voxel_colors_next.release();
     sc->bounds_work.release();
     delete sc;
     return VRT_OK;
@@ -679,7 +775,7 @@ int check_render_args(const vrt_scene* sc, const vrt_camera* cam, const vrt_rend
     if (cam && !p->use_samples && p->spp != 1)
         return fail(VRT_ERR_INVALID, std::string(who) + ": the temporal-blend mode renders one sample per frame (raycaster.hpp:77-85)");
     if (p->tile_step > 1 && (p->tile_index < 0 || p->tile_index >= p->tile_step)) return fail(VRT_ERR_INVALID, std::string(who) + ": tile_index must be in [0, tile_step)");
-    if (cam && !sc->has_tex) return fail(VRT_ERR_INVALID, std::string(who) + ": call vrt_scene_set_textures first (raycaster.hpp:53-54)");
+    if (cam && !sc->has_tex && !sc->has_palette) return fail(VRT_ERR_INVALID, std::string(who) + ": call vrt_scene_set_textures first (raycaster.hpp:53-54)");
     if (cam)    // a rotation (camera_controller.hpp:27-32): the frame kernels rely on |ray direction| staying near 1 (Trav2, kUnit)
         for (int i = 0; i < 9; ++i)
             if (!(std::fabs(cam->rot_mat[i]) <= 1024.0f)) return fail(VRT_ERR_INVALID, std::string(who) + ": rot_mat is not a rotation matrix");
@@ -690,6 +786,8 @@ int check_render_args(const vrt_scene* sc, const vrt_camera* cam, const vrt_rend
         if (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3)
             return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": mirror reflections need the reference node layout and render_variant 0, 2 or 4");
     }
+    if (cam && sc->has_palette && (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3))
+        return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": palette frames need the reference node layout and render_variant 0, 2 or 4");
     if (cam && p->autofocus && sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": autofocus needs an LSVO scene");
     if (cam && p->checker && sc->kind == VRT_SCENE_LSVO && (sc->ctx->render_variant == 1 || sc->ctx->render_variant >= 3))
         return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": the checkerboard needs render_variant 0 or 2");
@@ -719,6 +817,7 @@ vrt::RenderLaunch make_launch(const vrt_scene* sc, const vrt_camera* cam, const 
     L.roughness = p->roughness;
     L.max_bounds = p->max_bounds;
     L.mirror_y1 = sc->kind == VRT_SCENE_LSVO ? p->mirror_y1 : 0;
+    L.palette = sc->has_palette ? 1 : 0;
     L.checker = p->checker; L.checker_area_height = p->checker_area_height;
     L.focal = p->autofocus ? reinterpret_cast<const float*>(sc->d_counters + kFocalSlot) : nullptr;
     L.tile_step = p->tile_step > 1 ? p->tile_step : 1;
@@ -731,11 +830,26 @@ vrt::RenderLaunch make_launch(const vrt_scene* sc, const vrt_camera* cam, const 
 int vrt_scene_set_textures(vrt_scene* sc, const uint8_t* top_rgb, const uint8_t* side_rgb) {
     if (!sc || !top_rgb || !side_rgb) return fail(VRT_ERR_INVALID, "vrt_scene_set_textures: NULL argument");
     if (int s = use_device(sc->ctx)) return s;
-    if (!sc->d_tex) VRT_CUDA(cudaMalloc(&sc->d_tex, 1536));
+    if (!sc->d_tex) VRT_CUDA(cudaMalloc(&sc->d_tex, vrt::kTextureBlockBytes));
     VRT_CUDA(cudaMemcpyAsync(sc->d_tex, top_rgb, 768, cudaMemcpyHostToDevice, sc->ctx->stream));
     VRT_CUDA(cudaMemcpyAsync(sc->d_tex + 768, side_rgb, 768, cudaMemcpyHostToDevice, sc->ctx->stream));
     VRT_CUDA(cudaStreamSynchronize(sc->ctx->stream));
     sc->has_tex = true;
+    return VRT_OK;
+}
+
+int vrt_scene_set_palette(vrt_scene* sc, const uint8_t* rgb) {
+    if (!sc) return fail(VRT_ERR_INVALID, "vrt_scene_set_palette: scene is NULL");
+    if (sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, "vrt_scene_set_palette: needs an LSVO scene");
+    if (!rgb) {
+        sc->has_palette = false;
+        return VRT_OK;
+    }
+    if (int s = use_device(sc->ctx)) return s;
+    if (!sc->d_tex) VRT_CUDA(cudaMalloc(&sc->d_tex, vrt::kTextureBlockBytes));
+    VRT_CUDA(cudaMemcpyAsync(sc->d_tex + vrt::kPaletteOffset, rgb, 768, cudaMemcpyHostToDevice, sc->ctx->stream));
+    VRT_CUDA(cudaStreamSynchronize(sc->ctx->stream));
+    sc->has_palette = true;
     return VRT_OK;
 }
 
@@ -818,7 +932,7 @@ int vrt_render_resolve_device(vrt_scene* sc, const vrt_render_params* p, const u
 int vrt_shade_rays(vrt_scene* sc, const vrt_render_params* p, uint64_t n, const vrt_shade_job* jobs, vrt_shade_result* out) {
     if (!sc || !p) return fail(VRT_ERR_INVALID, "vrt_shade_rays: NULL argument");
     if (sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, "vrt_shade_rays: needs an LSVO scene");
-    if (!sc->has_tex) return fail(VRT_ERR_INVALID, "vrt_shade_rays: call vrt_scene_set_textures first (raycaster.hpp:53-54)");
+    if (!sc->has_tex && !sc->has_palette) return fail(VRT_ERR_INVALID, "vrt_shade_rays: call vrt_scene_set_textures first (raycaster.hpp:53-54)");
     if (p->gi_bounces < 0 || p->gi_bounces > 2) return fail(VRT_ERR_INVALID, "vrt_shade_rays: gi_bounces must be 0..2");
     if (n == 0) return VRT_OK;
     if (!jobs || !out) return fail(VRT_ERR_INVALID, "vrt_shade_rays: NULL buffer");
@@ -835,7 +949,8 @@ int vrt_shade_rays(vrt_scene* sc, const vrt_render_params* p, uint64_t n, const 
     vrt_render_params q = *p;
     if (q.width <= 0) q.width = 1;
     if (q.height <= 0) q.height = 1;
-    VRT_CUDA(vrt::launch_shade_rays(sc->use_compact ? sc->d_compact : sc->d_nodes, sc->use_compact, make_launch(sc, &cam, &q), n, d_jobs, d_out, ctx->stream));
+    const bool compact = sc->use_compact && !sc->has_palette;   // the palette instance reads colours from the reference array
+    VRT_CUDA(vrt::launch_shade_rays(compact ? sc->d_compact : sc->d_nodes, compact, make_launch(sc, &cam, &q), n, d_jobs, d_out, ctx->stream));
     ctx->launches += 1;
     VRT_CUDA(cudaMemcpyAsync(out, d_out, size_t(n) * sizeof(vrt_shade_result), cudaMemcpyDeviceToHost, ctx->stream));
     VRT_CUDA(cudaStreamSynchronize(ctx->stream));

@@ -83,8 +83,12 @@ struct vrt_scene {
     DeviceBuffer edit_old, bounds_work;         // staged rectangle of an edit; work memory of the scene-bounds sweep
     uint64_t* d_voxel_keys = nullptr;           // voxel-set scenes: sorted distinct path keys, resident for edits
     uint32_t n_voxel_keys = 0;
-    uint8_t* d_tex = nullptr;                   // top (768 B) then side (768 B)
+    // voxel-set scenes once painted: the colour of each resident key (it survives set_cells); an edit gathers the colours of the
+    // new key set into the second buffer and swaps the two, so that edits of a painted scene allocate nothing in the steady state
+    DeviceBuffer voxel_colors, voxel_colors_next;
+    uint8_t* d_tex = nullptr;                   // kTextureBlockBytes: top (768 B), side (768 B), palette (768 B)
     bool has_tex = false;
+    bool has_palette = false;                   // LSVO: frames take the albedo from the palette (vrt_scene_set_palette)
     DeviceBuffer frame_accum, frame_rgba;       // vrt_render staging
     DeviceBuffer frame_lists;                   // K6: sorted sample lists of the frame in flight
     DeviceBuffer beam_floor;                    // per-tile start distances of the camera rays of the frame in flight

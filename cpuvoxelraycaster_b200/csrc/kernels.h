@@ -76,10 +76,18 @@ struct RenderLaunch {
     float roughness;           // grid frames: blur of mirror reflections
     int max_bounds;            // reflection depth (RayCaster::max_bounds, raycaster.hpp:277)
     int mirror_y1;             // LSVO frames: 1 + y of the voxel layer whose top faces are Cell::Mirror; 0 = none
-    const float* focal;        // device: focal length computed by the autofocus kernel, or null = cam.focal_length
+    // LSVO frames (kMirror kernels) and shade rays: 1 = albedo = palette[colour of the hit voxel's leaf slot], the 256 RGB entries
+    // at tex_top + kPaletteOffset; 0 = the textures.  A flag in the alignment gap before `focal` rather than a pointer at the
+    // end: the struct keeps its 272 bytes, so no kernel parameter behind it moves.
+    int palette;
+    const float* focal;       // device: focal length computed by the autofocus kernel, or null = cam.focal_length
     int checker;               // 0 = every pixel, 1 / 2 = checkerboard with offset 0 / 1 (main.cpp:137,143)
     int checker_area_height;   // thread-area height the checkerboard phase restarts at (0 = never)
 };
+
+// A scene's texture block on the device: top texture, side texture (16x16 RGB each), then the 256-entry RGB palette.
+constexpr size_t kPaletteOffset = 1536;
+constexpr size_t kTextureBlockBytes = kPaletteOffset + 768;
 
 // main.cpp:143: inside a thread area, rows start at area_start + (x + offset) % 2 and step by 2.
 // Returns the parity x must have for pixel (x, y) to be rendered this frame.
@@ -189,4 +197,18 @@ cudaError_t device_edit_voxel_keys(const uint64_t* d_keys, uint32_t n_keys, cons
 cudaError_t device_build_lsvo_from_keys(int depth, const uint64_t* d_keys, uint32_t n_keys, uint2** d_slots, uint64_t* n_slots,
                                         cudaStream_t stream, BuildPool* pool = nullptr, uint64_t* capacity_slots = nullptr);
 cudaError_t device_compact_lsvo(const uint2* d_ref, uint64_t n_ref, int depth, uint2** d_out, uint64_t* n_out, cudaStream_t stream);
+// Per-voxel colours (voxel_build.cu), the `color` byte of each solid voxel's leaf slot in the reference layout.
+// Paints d_colors[i] into voxel d_xyz[i] (setCell coordinates); empty voxels are skipped, the last occurrence of a voxel wins.
+// d_keys / d_key_colors (optional, voxel-set scenes): the resident sorted keys and their colours, updated alongside.
+// *painted = distinct solid voxels painted.  Synchronises the stream.
+cudaError_t device_paint_cells(uint2* d_nodes, int depth, const uint32_t* d_xyz, const uint8_t* d_colors, uint64_t n,
+                               const uint64_t* d_keys, uint32_t n_keys, uint8_t* d_key_colors, uint64_t* painted, cudaStream_t stream);
+// d_out[i] = colour of voxel d_xyz[i], or -1 when it is empty
+cudaError_t launch_cell_colors(const uint2* d_nodes, int depth, const uint32_t* d_xyz, uint64_t n, int16_t* d_out, cudaStream_t stream);
+// Colours of a new sorted key set: the colour of the same key in the old set, else 1 (LNode())
+cudaError_t launch_gather_key_colors(const uint64_t* d_old_keys, const uint8_t* d_old_colors, uint32_t n_old, const uint64_t* d_new_keys,
+                                     uint32_t n_new, uint8_t* d_new_colors, cudaStream_t stream);
+// Writes the colour of every key into its leaf slot of a node array built from those keys
+cudaError_t launch_stamp_key_colors(uint2* d_nodes, int depth, const uint64_t* d_keys, const uint8_t* d_colors, uint32_t n_keys,
+                                    cudaStream_t stream);
 }  // namespace vrt

@@ -53,6 +53,24 @@ struct CompactNodes {
     }
 };
 
+// Leaf slot of voxel (x, y, z) in SVO::setCell coordinates (svo.hpp:72) in the reference layout: the root-to-leaf descent of
+// LSVO::getAtRayHit (lsvo.hpp:174-285), which returns node N and child slot s of the leaf; the leaf's own slot is
+// N + child_offset + s.  A voxel that castRay reports at v lies at S-1-v in these coordinates (SURVEY.md §0 item 2), so
+// the child slot is built from the coordinate bits directly.  kNoLeafSlot when a child bit on the way is missing (empty).
+// Only interior slots are loaded.
+constexpr uint32_t kNoLeafSlot = 0xffffffffu;
+__device__ __forceinline__ uint32_t lsvo_leaf_slot(const uint2* __restrict__ nodes, int depth, uint32_t x, uint32_t y, uint32_t z) {
+    uint32_t node = 0u;
+    for (int b = depth - 1; b >= 0; --b) {
+        const uint32_t slot = ((x >> b) & 1u) | (((y >> b) & 1u) << 1) | (((z >> b) & 1u) << 2);
+        const uint2 w = __ldg(nodes + node);
+        if (!((w.x >> (8 + slot)) & 1u)) return kNoLeafSlot;
+        node += w.y + slot;
+        if ((w.x >> (16 + slot)) & 1u) return node;
+    }
+    return kNoLeafSlot;
+}
+
 // Traversal state at termination (what the epilogue needs).
 struct LsvoResult {
     float px, py, pz;      // cell low corner in the mirrored frame (un-mirrored by lsvo_finish)

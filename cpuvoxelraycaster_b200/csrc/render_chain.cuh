@@ -108,9 +108,13 @@ __device__ __forceinline__ float lattice_dim(const RenderLaunch& L, uint32_t pix
 // The ray of stage `stage` ended with result (r, h).  Returns the next stage and, unless it is kDone, the next ray.
 // kMirror: mirror reflections on LSVO frames (extension specified in oracle/port.c, shade_sample): the top faces of the voxel
 // layer y = L.mirror_y1 - 1 are Cell::Mirror; a mirror hit re-enters kPrimary with the reflected, roughness-jittered ray.
-template <bool kMirror = false>
+// kPalette: with L.palette set, the albedo of the primary hit is the palette entry of the hit voxel's colour, read from its leaf
+// slot in `ref_nodes` (the reference layout; extension specified in tests/palette_oracle.c).  The frame kernels have it
+// with kMirror: mirror_y1 = 0 matches no face and the tint stays 1.
+template <bool kMirror = false, bool kPalette = kMirror>
 __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& c, int stage, const LsvoResult& r, const LsvoHit& h,
-                                             uint32_t pixel, uint32_t sample, float SCALE, float n_norm, NextRay& nr) {
+                                             uint32_t pixel, uint32_t sample, float SCALE, float n_norm, NextRay& nr,
+                                             const uint2* __restrict__ ref_nodes = nullptr) {
     nr.t_floor = 0.0f;                                                     // only camera rays have a beam floor
     switch (stage) {
         case kPrimary: {                                                   // raycaster.hpp:131-145
@@ -135,11 +139,22 @@ __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& 
             }
             c.have_hit = true;
             c.nx = h.normal[0]; c.ny = h.normal[1]; c.nz = h.normal[2];
-            const uint8_t* tex = (c.ny != 0.0f) ? L.tex_top : L.tex_side;  // :211-215
-            const float u = fminf(fmaxf(h.uv[0], 0.0f), 1.0f), v = fminf(fmaxf(h.uv[1], 0.0f), 1.0f);   // :237-238
-            const uint32_t tx = uint32_t(16.0f * u), ty = uint32_t(16.0f * v);                          // :239
-            const uint8_t* texel = tex + 3u * (ty * 16u + tx);
-            c.tex_r = __ldg(texel); c.tex_g = __ldg(texel + 1); c.tex_b = __ldg(texel + 2);
+            if (kPalette && L.palette) {
+                // castRay voxel v = setCell coordinate S-1-v, taken from the hit cell's corner like the mirror test above
+                const float S = float(1 << L.depth);
+                const uint32_t S1 = (1u << L.depth) - 1u;
+                const uint32_t slot = lsvo_leaf_slot(ref_nodes, L.depth, S1 - uint32_t(int((h.corner[0] - 1.0f) * S)),
+                                                     S1 - uint32_t(int((h.corner[1] - 1.0f) * S)), S1 - uint32_t(int((h.corner[2] - 1.0f) * S)));
+                const uint32_t colour = slot != kNoLeafSlot ? (__ldg(ref_nodes + slot).x & 0xffu) : 1u;
+                const uint8_t* entry = L.tex_top + kPaletteOffset + 3u * colour;
+                c.tex_r = __ldg(entry); c.tex_g = __ldg(entry + 1); c.tex_b = __ldg(entry + 2);
+            } else {
+                const uint8_t* tex = (c.ny != 0.0f) ? L.tex_top : L.tex_side;  // :211-215
+                const float u = fminf(fmaxf(h.uv[0], 0.0f), 1.0f), v = fminf(fmaxf(h.uv[1], 0.0f), 1.0f);   // :237-238
+                const uint32_t tx = uint32_t(16.0f * u), ty = uint32_t(16.0f * v);                          // :239
+                const uint8_t* texel = tex + 3u * (ty * 16u + tx);
+                c.tex_r = __ldg(texel); c.tex_g = __ldg(texel + 1); c.tex_b = __ldg(texel + 2);
+            }
             c.gpx = h.pos[0]; c.gpy = h.pos[1]; c.gpz = h.pos[2];         // the GI stage starts from the primary hit
             nr.ox = h.pos[0] + c.nx * SCALE * 0.001f;                      // sun shadow ray, :139
             nr.oy = h.pos[1] + c.ny * SCALE * 0.001f;

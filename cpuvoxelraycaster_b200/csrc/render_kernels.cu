@@ -97,7 +97,7 @@ __global__ void __launch_bounds__(128, VRT_K4_MIN_CTAS) render_accumulate_kernel
                     stack.stat_add(stage, 1u, r.complexity);
                     LsvoHit h;
                     if (r.hit) lsvo_finish(r, nr.ox, nr.oy, nr.oz, L.depth, h);
-                    stage = chain_advance<kMirror>(L, c, stage, r, h, pixel, sample, SCALE, n_norm, nr);
+                    stage = chain_advance<kMirror>(L, c, stage, r, h, pixel, sample, SCALE, n_norm, nr, nodes.slots);
                 }
                 chain_colour<kMirror>(L, c, sum_r, sum_g, sum_b);
             }
@@ -521,7 +521,7 @@ __global__ void __launch_bounds__(128, VRT_K6_MIN_CTAS) render_rounds_kernel(Nod
                     stack2.stat_add(stage, 1u, r.complexity);
                     LsvoHit h;
                     if (r.hit) lsvo_finish(r, nr.ox, nr.oy, nr.oz, L.depth, h);
-                    stage = chain_advance<kMirror>(L, cs, stage, r, h, pixel, sample, SCALE, n_norm, nr);
+                    stage = chain_advance<kMirror>(L, cs, stage, r, h, pixel, sample, SCALE, n_norm, nr, nodes.slots);
                 }
                 chain_colour<kMirror>(L, cs, cr, cg, cb);
             }
@@ -615,7 +615,8 @@ __global__ void __launch_bounds__(128, VRT_K6_MIN_CTAS) render_rounds_kernel(Nod
 // reference's renderRay receives from Camera::getRay (main.cpp:147-149) — and gets the sample's colour back.  One thread per
 // ray, the same sample chain as the frame kernels (sun shadow, GI with the Philox numbers of (pixel, sample)), so a ray
 // that equals the frame kernels' primary ray of (pixel, sample) gives exactly that sample's colour.
-template <typename Nodes, bool kGuard>
+// kPalette: albedo from the scene's palette (L.palette); `nodes` is then the reference layout.
+template <typename Nodes, bool kGuard, bool kPalette = false>
 __global__ void __launch_bounds__(128, 8) shade_rays_kernel(Nodes nodes, RenderLaunch L, uint64_t n, const vrt_shade_job* __restrict__ jobs,
                                                          vrt_shade_result* __restrict__ out) {
     extern __shared__ uint2 smem[];
@@ -648,7 +649,7 @@ __global__ void __launch_bounds__(128, 8) shade_rays_kernel(Nodes nodes, RenderL
         if (stage == kPrimary) { complexity = r.complexity; if (r.hit) distance = r.t_min; }   // RayContext, raycaster.hpp:132-133,137
         LsvoHit h;
         if (r.hit) lsvo_finish(r, nr.ox, nr.oy, nr.oz, L.depth, h);
-        stage = chain_advance(L, c, stage, r, h, job.pixel, job.sample, SCALE, n_norm, nr);
+        stage = chain_advance<false, kPalette>(L, c, stage, r, h, job.pixel, job.sample, SCALE, n_norm, nr, nodes.slots);
     }
     uint32_t cr = 0, cg = 0, cb = 0;
     chain_colour(L, c, cr, cg, cb);
@@ -665,7 +666,9 @@ cudaError_t launch_shade_rays(const uint2* nodes, bool compact, const RenderLaun
     if (!n) return cudaSuccess;
     const size_t smem = size_t(L.depth + 1) * 128 * 8;
     const unsigned grid = unsigned((n + 127) / 128);
-    if (compact) shade_rays_kernel<CompactNodes, true><<<grid, 128, smem, stream>>>(CompactNodes{nodes}, L, n, d_jobs, d_out);
+    // palette: `nodes` is the reference array whatever the scene's layout (the colours live in its leaf slots)
+    if (L.palette) shade_rays_kernel<RefNodes, true, true><<<grid, 128, smem, stream>>>(RefNodes{nodes}, L, n, d_jobs, d_out);
+    else if (compact) shade_rays_kernel<CompactNodes, true><<<grid, 128, smem, stream>>>(CompactNodes{nodes}, L, n, d_jobs, d_out);
     else if (guard_binds(L)) shade_rays_kernel<RefNodes, true><<<grid, 128, smem, stream>>>(RefNodes{nodes}, L, n, d_jobs, d_out);
     else shade_rays_kernel<RefNodes, false><<<grid, 128, smem, stream>>>(RefNodes{nodes}, L, n, d_jobs, d_out);
     return cudaGetLastError();
@@ -790,7 +793,7 @@ cudaError_t launch_render_accumulate_ref(const uint2* nodes, bool compact, const
             kernel<<<grid6, block, smem, stream>>>(view, L, P.G, lists, meta, d_accum, d_counters);
         };
         if (compact) launch6(render_rounds_kernel<CompactNodes, 0>, CompactNodes{nodes});
-        else if (L.mirror_y1 > 0) {
+        else if (L.mirror_y1 > 0 || L.palette) {
             if (guard_binds(L)) launch6(render_rounds_kernel<RefNodes, 2, true, true>, RefNodes{nodes});
             else launch6(render_rounds_kernel<RefNodes, 2, true, false>, RefNodes{nodes});
         } else switch (L.trav_policy) {
@@ -855,7 +858,7 @@ cudaError_t launch_render_accumulate_ref(const uint2* nodes, bool compact, const
     if (compact) {
         if (live) launch4(render_accumulate_kernel<CompactNodes, true>, CompactNodes{nodes});
         else launch4(render_accumulate_kernel<CompactNodes, false>, CompactNodes{nodes});
-    } else if (L.mirror_y1 > 0) {
+    } else if (L.mirror_y1 > 0 || L.palette) {
         if (live) { if (guarded) launch4(render_accumulate_kernel<RefNodes, true, true, true>, RefNodes{nodes}); else launch4(render_accumulate_kernel<RefNodes, true, true, false>, RefNodes{nodes}); }
         else { if (guarded) launch4(render_accumulate_kernel<RefNodes, false, true, true>, RefNodes{nodes}); else launch4(render_accumulate_kernel<RefNodes, false, true, false>, RefNodes{nodes}); }
     } else {

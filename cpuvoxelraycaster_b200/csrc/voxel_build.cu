@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "kernels.h"
+#include "lsvo_traverse.cuh"
 
 namespace vrt {
 
@@ -141,7 +142,127 @@ cudaError_t sort_unique(uint64_t* d_in, uint32_t n, int bits, uint64_t* d_sorted
     return cudaStreamSynchronize(stream);
 }
 
+// ---- per-voxel colours: the `color` byte of a solid voxel's leaf slot (DESIGN.md §2) ----------------------------------------
+__device__ __forceinline__ uint64_t voxel_key(uint32_t x, uint32_t y, uint32_t z, int depth) {     // as voxel_keys_kernel
+    uint64_t key = 0;
+    for (int b = depth - 1; b >= 0; --b)
+        key = (key << 3) | uint64_t((((x >> b) & 1u) << 2) | (((y >> b) & 1u) << 1) | ((z >> b) & 1u));
+    return key;
+}
+
+// slot[i] = leaf slot of voxel i (kNoLeafSlot when empty), index[i] = i
+__global__ void paint_slots_kernel(const uint2* __restrict__ nodes, int depth, const uint32_t* __restrict__ xyz, uint32_t n,
+                                   uint32_t* __restrict__ slot, uint32_t* __restrict__ index) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    slot[i] = lsvo_leaf_slot(nodes, depth, xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]);
+    index[i] = i;
+}
+
+// (slot, index) pairs sorted by slot, stably: the last entry of a run of equal slots is the voxel's last occurrence in the list
+__global__ void paint_write_kernel(uint2* __restrict__ nodes, int depth, const uint32_t* __restrict__ xyz, const uint8_t* __restrict__ colors,
+                                   const uint32_t* __restrict__ slot, const uint32_t* __restrict__ index, uint32_t n,
+                                   const uint64_t* __restrict__ keys, uint32_t n_keys, uint8_t* __restrict__ key_colors,
+                                   unsigned long long* __restrict__ painted) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const uint32_t s = slot[j];
+    if (s == kNoLeafSlot || (j + 1 < n && slot[j + 1] == s)) return;
+    const uint32_t i = index[j];
+    const uint8_t c = colors[i];
+    reinterpret_cast<uint8_t*>(nodes + s)[0] = c;                           // LNode::color, lsvo_utils.hpp:14
+    if (key_colors) {
+        const uint64_t key = voxel_key(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2], depth);
+        key_colors[lower_bound_u64(keys, n_keys, key)] = c;                  // solid: the key is resident
+    }
+    atomicAdd(painted, 1ull);
+}
+
+__global__ void cell_colors_kernel(const uint2* __restrict__ nodes, int depth, const uint32_t* __restrict__ xyz, uint64_t n,
+                                   int16_t* __restrict__ out) {
+    const uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t s = lsvo_leaf_slot(nodes, depth, xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]);
+    out[i] = s == kNoLeafSlot ? int16_t(-1) : int16_t(__ldg(nodes + s).x & 0xffu);
+}
+
+__global__ void gather_key_colors_kernel(const uint64_t* __restrict__ old_keys, const uint8_t* __restrict__ old_colors, uint32_t n_old,
+                                         const uint64_t* __restrict__ new_keys, uint32_t n_new, uint8_t* __restrict__ new_colors) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_new) return;
+    const uint64_t key = new_keys[j];
+    const uint32_t k = lower_bound_u64(old_keys, n_old, key);
+    new_colors[j] = (k < n_old && old_keys[k] == key) ? old_colors[k] : uint8_t(1);    // added voxels: LNode() colour
+}
+
+__global__ void stamp_key_colors_kernel(uint2* __restrict__ nodes, int depth, const uint64_t* __restrict__ keys,
+                                        const uint8_t* __restrict__ colors, uint32_t n_keys) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_keys) return;
+    const uint64_t key = keys[j];
+    uint32_t x = 0, y = 0, z = 0;
+    for (int b = depth - 1; b >= 0; --b) {
+        const uint32_t d = uint32_t(key >> (3 * b)) & 7u;
+        x |= (d >> 2) << b; y |= ((d >> 1) & 1u) << b; z |= (d & 1u) << b;
+    }
+    const uint32_t s = lsvo_leaf_slot(nodes, depth, x, y, z);
+    if (s != kNoLeafSlot) reinterpret_cast<uint8_t*>(nodes + s)[0] = colors[j];
+}
+
 }  // namespace
+
+cudaError_t device_paint_cells(uint2* d_nodes, int depth, const uint32_t* d_xyz, const uint8_t* d_colors, uint64_t n,
+                               const uint64_t* d_keys, uint32_t n_keys, uint8_t* d_key_colors, uint64_t* painted, cudaStream_t stream) {
+    *painted = 0;
+    if (n == 0) return cudaSuccess;
+    if (n > 0x7fffffffull) return cudaErrorInvalidValue;
+    const uint32_t m = uint32_t(n);
+    Scratch sc(nullptr);
+    uint32_t *slot = nullptr, *index = nullptr, *slot_sorted = nullptr, *index_sorted = nullptr;
+    unsigned long long* d_count = nullptr;
+    VRT_TRY(sc.alloc(&slot, m));
+    VRT_TRY(sc.alloc(&index, m));
+    VRT_TRY(sc.alloc(&slot_sorted, m));
+    VRT_TRY(sc.alloc(&index_sorted, m));
+    VRT_TRY(sc.alloc(&d_count, 1));
+    size_t t = 0;
+    VRT_TRY(cub::DeviceRadixSort::SortPairs(nullptr, t, slot, slot_sorted, index, index_sorted, m, 0, 32, stream));
+    uint8_t* d_temp = nullptr;
+    VRT_TRY(sc.alloc(&d_temp, t));
+    VRT_TRY(cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), stream));
+    const unsigned blocks = (m + 255) / 256;
+    paint_slots_kernel<<<blocks, 256, 0, stream>>>(d_nodes, depth, d_xyz, m, slot, index);
+    VRT_TRY(cudaGetLastError());
+    VRT_TRY(cub::DeviceRadixSort::SortPairs(d_temp, t, slot, slot_sorted, index, index_sorted, m, 0, 32, stream));   // LSD radix: stable
+    paint_write_kernel<<<blocks, 256, 0, stream>>>(d_nodes, depth, d_xyz, d_colors, slot_sorted, index_sorted, m, d_keys, n_keys,
+                                                   d_key_colors, d_count);
+    VRT_TRY(cudaGetLastError());
+    unsigned long long count = 0;
+    VRT_TRY(cudaMemcpyAsync(&count, d_count, sizeof(count), cudaMemcpyDeviceToHost, stream));
+    VRT_TRY(cudaStreamSynchronize(stream));
+    *painted = count;
+    return cudaSuccess;
+}
+
+cudaError_t launch_cell_colors(const uint2* d_nodes, int depth, const uint32_t* d_xyz, uint64_t n, int16_t* d_out, cudaStream_t stream) {
+    if (n == 0) return cudaSuccess;
+    cell_colors_kernel<<<unsigned((n + 255) / 256), 256, 0, stream>>>(d_nodes, depth, d_xyz, n, d_out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_gather_key_colors(const uint64_t* d_old_keys, const uint8_t* d_old_colors, uint32_t n_old, const uint64_t* d_new_keys,
+                                     uint32_t n_new, uint8_t* d_new_colors, cudaStream_t stream) {
+    if (n_new == 0) return cudaSuccess;
+    gather_key_colors_kernel<<<(n_new + 255) / 256, 256, 0, stream>>>(d_old_keys, d_old_colors, n_old, d_new_keys, n_new, d_new_colors);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_stamp_key_colors(uint2* d_nodes, int depth, const uint64_t* d_keys, const uint8_t* d_colors, uint32_t n_keys,
+                                    cudaStream_t stream) {
+    if (n_keys == 0) return cudaSuccess;
+    stamp_key_colors_kernel<<<(n_keys + 255) / 256, 256, 0, stream>>>(d_nodes, depth, d_keys, d_colors, n_keys);
+    return cudaGetLastError();
+}
 
 // xyz (device, n triples, coordinates < 2^depth) → sorted distinct voxel keys.  *d_keys is cudaMalloc'ed (caller frees).
 cudaError_t device_voxel_keys(const uint32_t* d_xyz, uint64_t n, int depth, uint64_t** d_keys, uint32_t* n_keys, cudaStream_t stream,

@@ -260,21 +260,53 @@ class LSVO(Volumetric):
         return nodes
 
     @classmethod
-    def from_voxels(cls, ctx, depth, xyz, guard=0, on_device=False):
+    def from_voxels(cls, ctx, depth, xyz, guard=0, on_device=False, colors=None):
         """SVO::setCell for every voxel (svo.hpp:72) followed by LSVO(const SVO&) (lsvo.hpp:12).  on_device=True: the
-        voxel list is flattened on the GPU (byte-identical) and stays editable through set_cells."""
+        voxel list is flattened on the GPU (byte-identical) and stays editable through set_cells.  colors (uint8 per voxel,
+        optional): painted afterwards (paint_cells)."""
         if not on_device:
-            return cls(ctx, host_build_lsvo_from_voxels(depth, xyz), depth, guard)
-        v = np.ascontiguousarray(np.asarray(xyz, np.uint32).reshape(-1, 3))
-        self = cls.__new__(cls)
-        Volumetric.__init__(self, ctx)
-        h = C.c_void_p()
-        check(lib().vrt_lsvo_create_from_voxels(ctx.handle, int(depth), ptr(v) if len(v) else None, len(v), int(guard), C.byref(h)))
-        self.handle = h
-        self.depth = int(depth)
-        self.n_nodes = len(self)
-        self._layout_from_env()
+            self = cls(ctx, host_build_lsvo_from_voxels(depth, xyz), depth, guard)
+        else:
+            v = np.ascontiguousarray(np.asarray(xyz, np.uint32).reshape(-1, 3))
+            self = cls.__new__(cls)
+            Volumetric.__init__(self, ctx)
+            h = C.c_void_p()
+            check(lib().vrt_lsvo_create_from_voxels(ctx.handle, int(depth), ptr(v) if len(v) else None, len(v), int(guard), C.byref(h)))
+            self.handle = h
+            self.depth = int(depth)
+            self.n_nodes = len(self)
+            self._layout_from_env()
+        if colors is not None:
+            self.paint_cells(xyz, colors)
         return self
+
+    def paint_cells(self, xyz, colors):
+        """Per-voxel colours (extension): sets the `color` byte of the leaf slots of the solid voxels xyz (setCell
+        coordinates).  Empty voxels are skipped; a voxel listed twice takes its last colour.  Returns the number of distinct
+        solid voxels painted.  Frames show the colours through set_palette."""
+        v = np.ascontiguousarray(np.asarray(xyz, np.uint32).reshape(-1, 3))
+        c = np.ascontiguousarray(np.broadcast_to(np.asarray(colors, np.uint8), (len(v),)))
+        n = C.c_uint64(0)
+        check(lib().vrt_scene_paint_cells(self.handle, ptr(v) if len(v) else None, ptr(c) if len(v) else None, len(v), C.byref(n)))
+        return int(n.value)
+
+    def cell_colors(self, xyz):
+        """int16 per voxel: its colour, or -1 where the voxel is empty."""
+        v = np.ascontiguousarray(np.asarray(xyz, np.uint32).reshape(-1, 3))
+        out = np.zeros(len(v), np.int16)
+        check(lib().vrt_scene_cell_colors(self.handle, ptr(v) if len(v) else None, len(v), ptr(out) if len(v) else None))
+        return out
+
+    def set_palette(self, rgb):
+        """rgb: uint8 [256, 3] (entry c is the albedo of colour c) — frames take the albedo from it instead of the textures;
+        None = back to the textures."""
+        if rgb is None:
+            check(lib().vrt_scene_set_palette(self.handle, None))
+            return
+        p = np.ascontiguousarray(rgb, np.uint8)
+        if p.size != 768:
+            raise ValueError("the palette must be 256 RGB entries")
+        check(lib().vrt_scene_set_palette(self.handle, ptr(p)))
 
     def set_cells(self, xyz, solid=True):
         """Dynamic scene: adds (solid) or removes voxels of a from_voxels(on_device=True) world and re-flattens it on

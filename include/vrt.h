@@ -171,6 +171,16 @@ int vrt_scene_voxel_count(const vrt_scene* scene, uint64_t* count);
 int vrt_lsvo_create_heightfield(vrt_context* ctx, uint32_t depth, const int32_t* heights, int32_t guard, vrt_scene** out);
 int vrt_scene_edit_heights(vrt_scene* scene, uint32_t x0, uint32_t z0, uint32_t nx, uint32_t nz, const int32_t* heights);
 int vrt_scene_download_heights(vrt_scene* scene, int32_t* heights /* [S*S] */);
+/* Per-voxel colours (extension, DESIGN.md §2).  A solid voxel's colour is the `color` byte of its leaf slot in the reference
+ * layout (lsvo_utils.hpp:5-18): data[node + child_offset + slot] for the node and slot LSVO::getAtRayHit finds.  Unpainted
+ * voxels keep LNode()'s 1.  Casts and textured frames never read it.  Accepted on scenes from vrt_lsvo_create,
+ * vrt_lsvo_create_terrain and vrt_lsvo_create_from_voxels (VRT_ERR_UNSUPPORTED for heightfield, grid and SVO scenes); on a
+ * voxel-set scene the colours survive vrt_scene_set_cells (added voxels get 1).
+ * Sets the colour of solid voxels (xyz in SVO::setCell coordinates, svo.hpp:72).  Empty voxels are skipped; when a voxel
+ * appears twice the last occurrence wins; *painted (may be NULL) = distinct solid voxels painted.  Synchronises the stream. */
+int vrt_scene_paint_cells(vrt_scene* scene, const uint32_t* xyz, const uint8_t* colors, uint64_t n, uint64_t* painted);
+/* out[i] = colour of voxel i, or -1 if it is empty. */
+int vrt_scene_cell_colors(vrt_scene* scene, const uint32_t* xyz, uint64_t n, int16_t* out);
 /* Device-side node layout of an LSVO scene (no reference counterpart; results are identical for both):
  *   0 = the reference's LNode array (default), 1 = compact breadth-first array of live nodes (8x smaller, built on the
  *   device on first use).  l2_persist != 0 additionally pins the front of the compact array (the top octree levels)
@@ -254,6 +264,11 @@ typedef struct vrt_render_stats {
  *
  * 16x16 RGB albedo textures, top-down rows: RayCaster::image_top / image_side (raycaster.hpp:53-54). */
 int vrt_scene_set_textures(vrt_scene* scene, const uint8_t* top_rgb, const uint8_t* side_rgb);
+/* LSVO scenes: while a palette is set, a sample's albedo is palette[colour of the voxel its camera ray hits] (the last,
+ * non-mirror hit) instead of the texel; shadows, GI, mirror tint and rounding stay as they are.  Frames then need no
+ * textures, the reference node layout and render_variant 0, 2 or 4 (VRT_ERR_UNSUPPORTED otherwise); vrt_shade_rays and
+ * vrt_render_distributed honour it.  rgb = 256*3 bytes (entry c is the albedo of colour c); NULL = back to the textures. */
+int vrt_scene_set_palette(vrt_scene* scene, const uint8_t* rgb);
 
 /* d_accum: device uint32 [height*width*4] r,g,b,count sums (RayCaster::colors, raycaster.hpp:259; the
  * integer sums equal the reference's double accumulators exactly).  Rows outside [row_begin,row_end)

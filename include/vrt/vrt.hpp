@@ -275,6 +275,27 @@ struct LSVO : public Volumetric {
         return nullptr;
     }
 
+    // Per-voxel colours (extension; the reference sets LNode::color to 1 and never reads it).  xyz: SVO::setCell triples.
+    // Paints the solid voxels (empty ones are skipped, the last occurrence of a voxel wins) and refreshes `data`, so that
+    // data[] and getAtRayHit show the colours.  Returns the number of distinct solid voxels painted.
+    uint64_t paintCells(const std::vector<uint32_t>& xyz, const std::vector<uint8_t>& colors) {
+        if (xyz.size() != 3 * colors.size()) throw vrt::Error(VRT_ERR_INVALID, "paintCells: one colour per xyz triple");
+        uint64_t painted = 0;
+        vrt::check(vrt_scene_paint_cells(m_scene.s, xyz.data(), colors.data(), colors.size(), &painted));
+        uint64_t n = data.size();
+        vrt::check(vrt_scene_download_nodes(m_scene.s, data.data(), data.size(), &n));
+        return painted;
+    }
+    // colour of each voxel, -1 where it is empty
+    std::vector<int16_t> getCellColors(const std::vector<uint32_t>& xyz) const {
+        std::vector<int16_t> out(xyz.size() / 3);
+        vrt::check(vrt_scene_cell_colors(m_scene.s, xyz.data(), out.size(), out.data()));
+        return out;
+    }
+    // frames take the albedo of colour c from rgb[3c..3c+2] (256 entries) instead of the textures, until clearPalette()
+    void setPalette(const uint8_t rgb[768]) { vrt::check(vrt_scene_set_palette(m_scene.s, rgb)); }
+    void clearPalette() { vrt::check(vrt_scene_set_palette(m_scene.s, nullptr)); }
+
     std::vector<vrt_lnode> data;                        // LNode[] in the reference layout (lsvo.hpp:287)
     const vrt_lnode* raw_data = nullptr;                // lsvo.hpp:288
     Cell* cell = nullptr;                               // the one shared Solid/Grass cell (lsvo.hpp:21-23,289)
