@@ -79,6 +79,7 @@ _SIGNATURES = {
     "vrt_scene_last_complexity": (C.c_int, [_vp, C.POINTER(_u64)]),
     "vrt_scene_set_textures": (C.c_int, [_vp, _vp, _vp]),
     "vrt_scene_set_palette": (C.c_int, [_vp, _vp]),
+    "vrt_scene_set_cell_types": (C.c_int, [_vp, _vp]),
     "vrt_scene_paint_cells": (C.c_int, [_vp, _vp, _vp, _u64, C.POINTER(_u64)]),
     "vrt_scene_cell_colors": (C.c_int, [_vp, _vp, _u64, _vp]),
     "vrt_render_accumulate_device": (C.c_int, [_vp, C.POINTER(Camera), C.POINTER(RenderParams), _vp]),

@@ -786,6 +786,11 @@ int check_render_args(const vrt_scene* sc, const vrt_camera* cam, const vrt_rend
         if (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3)
             return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": mirror reflections need the reference node layout and render_variant 0, 2 or 4");
     }
+    if (cam && sc->has_cell_types) {
+        if (p->max_bounds < 0 || p->max_bounds > 16) return fail(VRT_ERR_INVALID, std::string(who) + ": max_bounds must be 0..16");
+        if (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3)
+            return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": mirror voxels need the reference node layout and render_variant 0, 2 or 4");
+    }
     if (cam && sc->has_palette && (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3))
         return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": palette frames need the reference node layout and render_variant 0, 2 or 4");
     if (cam && p->autofocus && sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": autofocus needs an LSVO scene");
@@ -817,7 +822,7 @@ vrt::RenderLaunch make_launch(const vrt_scene* sc, const vrt_camera* cam, const 
     L.roughness = p->roughness;
     L.max_bounds = p->max_bounds;
     L.mirror_y1 = sc->kind == VRT_SCENE_LSVO ? p->mirror_y1 : 0;
-    L.palette = sc->has_palette ? 1 : 0;
+    L.palette = (sc->has_palette ? vrt::kPaletteAlbedo : 0) | (sc->has_cell_types ? vrt::kCellTypes : 0);
     L.checker = p->checker; L.checker_area_height = p->checker_area_height;
     L.focal = p->autofocus ? reinterpret_cast<const float*>(sc->d_counters + kFocalSlot) : nullptr;
     L.tile_step = p->tile_step > 1 ? p->tile_step : 1;
@@ -850,6 +855,29 @@ int vrt_scene_set_palette(vrt_scene* sc, const uint8_t* rgb) {
     VRT_CUDA(cudaMemcpyAsync(sc->d_tex + vrt::kPaletteOffset, rgb, 768, cudaMemcpyHostToDevice, sc->ctx->stream));
     VRT_CUDA(cudaStreamSynchronize(sc->ctx->stream));
     sc->has_palette = true;
+    return VRT_OK;
+}
+
+int vrt_scene_set_cell_types(vrt_scene* sc, const uint8_t* types) {
+    if (!sc) return fail(VRT_ERR_INVALID, "vrt_scene_set_cell_types: scene is NULL");
+    if (sc->kind != VRT_SCENE_LSVO)
+        return fail(VRT_ERR_UNSUPPORTED, "vrt_scene_set_cell_types: needs an LSVO scene (grid and SVO scenes have cell types of their own)");
+    bool mirror = false;
+    if (types)
+        for (int i = 0; i < 256; ++i) {
+            if (types[i] != 1 && types[i] != 2)
+                return fail(VRT_ERR_INVALID, "vrt_scene_set_cell_types: every entry must be 1 (Cell::Solid) or 2 (Cell::Mirror)");
+            mirror |= types[i] == 2;
+        }
+    if (!mirror) {                                            // all Solid: the frames of a scene without a table
+        sc->has_cell_types = false;
+        return VRT_OK;
+    }
+    if (int s = use_device(sc->ctx)) return s;
+    if (!sc->d_tex) VRT_CUDA(cudaMalloc(&sc->d_tex, vrt::kTextureBlockBytes));
+    VRT_CUDA(cudaMemcpyAsync(sc->d_tex + vrt::kCellTypesOffset, types, 256, cudaMemcpyHostToDevice, sc->ctx->stream));
+    VRT_CUDA(cudaStreamSynchronize(sc->ctx->stream));
+    sc->has_cell_types = true;
     return VRT_OK;
 }
 
@@ -934,6 +962,7 @@ int vrt_shade_rays(vrt_scene* sc, const vrt_render_params* p, uint64_t n, const 
     if (sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, "vrt_shade_rays: needs an LSVO scene");
     if (!sc->has_tex && !sc->has_palette) return fail(VRT_ERR_INVALID, "vrt_shade_rays: call vrt_scene_set_textures first (raycaster.hpp:53-54)");
     if (p->gi_bounces < 0 || p->gi_bounces > 2) return fail(VRT_ERR_INVALID, "vrt_shade_rays: gi_bounces must be 0..2");
+    if (sc->has_cell_types && (p->max_bounds < 0 || p->max_bounds > 16)) return fail(VRT_ERR_INVALID, "vrt_shade_rays: max_bounds must be 0..16");
     if (n == 0) return VRT_OK;
     if (!jobs || !out) return fail(VRT_ERR_INVALID, "vrt_shade_rays: NULL buffer");
     if (n > (1ull << 31)) return fail(VRT_ERR_UNSUPPORTED, "vrt_shade_rays: too many rays for one call");
@@ -949,7 +978,8 @@ int vrt_shade_rays(vrt_scene* sc, const vrt_render_params* p, uint64_t n, const 
     vrt_render_params q = *p;
     if (q.width <= 0) q.width = 1;
     if (q.height <= 0) q.height = 1;
-    const bool compact = sc->use_compact && !sc->has_palette;   // the palette instance reads colours from the reference array
+    // the palette instance reads colours from the reference array
+    const bool compact = sc->use_compact && !sc->has_palette && !sc->has_cell_types;
     VRT_CUDA(vrt::launch_shade_rays(compact ? sc->d_compact : sc->d_nodes, compact, make_launch(sc, &cam, &q), n, d_jobs, d_out, ctx->stream));
     ctx->launches += 1;
     VRT_CUDA(cudaMemcpyAsync(out, d_out, size_t(n) * sizeof(vrt_shade_result), cudaMemcpyDeviceToHost, ctx->stream));

@@ -76,18 +76,25 @@ struct RenderLaunch {
     float roughness;           // grid frames: blur of mirror reflections
     int max_bounds;            // reflection depth (RayCaster::max_bounds, raycaster.hpp:277)
     int mirror_y1;             // LSVO frames: 1 + y of the voxel layer whose top faces are Cell::Mirror; 0 = none
-    // LSVO frames (kMirror kernels) and shade rays: 1 = albedo = palette[colour of the hit voxel's leaf slot], the 256 RGB entries
-    // at tex_top + kPaletteOffset; 0 = the textures.  A flag in the alignment gap before `focal` rather than a pointer at the
-    // end: the struct keeps its 272 bytes, so no kernel parameter behind it moves.
+    // LSVO frames (kMirror kernels) and shade rays, a bit set over the colour of the hit voxel's leaf slot:
+    //   kPaletteAlbedo  albedo = palette[colour], the 256 RGB entries at tex_top + kPaletteOffset (else the textures)
+    //   kCellTypes      types[colour] == Cell::Mirror reflects camera-chain rays, the 256 bytes at tex_top + kCellTypesOffset
+    // Bits in the alignment gap before `focal` rather than pointers at the end: the struct keeps its 272 bytes, so no kernel
+    // parameter behind it moves.
     int palette;
     const float* focal;       // device: focal length computed by the autofocus kernel, or null = cam.focal_length
     int checker;               // 0 = every pixel, 1 / 2 = checkerboard with offset 0 / 1 (main.cpp:137,143)
     int checker_area_height;   // thread-area height the checkerboard phase restarts at (0 = never)
 };
 
-// A scene's texture block on the device: top texture, side texture (16x16 RGB each), then the 256-entry RGB palette.
+constexpr int kPaletteAlbedo = 1, kCellTypes = 2;
+static_assert(sizeof(RenderLaunch) == 272, "RenderLaunch is a kernel parameter of every frame kernel");
+
+// A scene's texture block on the device: top texture, side texture (16x16 RGB each), the 256-entry RGB palette, then the
+// 256 Cell::Type bytes of the colours (1 = Solid, 2 = Mirror).
 constexpr size_t kPaletteOffset = 1536;
-constexpr size_t kTextureBlockBytes = kPaletteOffset + 768;
+constexpr size_t kCellTypesOffset = kPaletteOffset + 768;
+constexpr size_t kTextureBlockBytes = kCellTypesOffset + 256;
 
 // main.cpp:143: inside a thread area, rows start at area_start + (x + offset) % 2 and step by 2.
 // Returns the parity x must have for pixel (x, y) to be rendered this frame.

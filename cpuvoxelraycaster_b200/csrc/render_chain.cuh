@@ -108,9 +108,10 @@ __device__ __forceinline__ float lattice_dim(const RenderLaunch& L, uint32_t pix
 // The ray of stage `stage` ended with result (r, h).  Returns the next stage and, unless it is kDone, the next ray.
 // kMirror: mirror reflections on LSVO frames (extension specified in oracle/port.c, shade_sample): the top faces of the voxel
 // layer y = L.mirror_y1 - 1 are Cell::Mirror; a mirror hit re-enters kPrimary with the reflected, roughness-jittered ray.
-// kPalette: with L.palette set, the albedo of the primary hit is the palette entry of the hit voxel's colour, read from its leaf
-// slot in `ref_nodes` (the reference layout; extension specified in tests/palette_oracle.c).  The frame kernels have it
-// with kMirror: mirror_y1 = 0 matches no face and the tint stays 1.
+// kPalette: L.palette's bits read the colour of the hit voxel from its leaf slot in `ref_nodes` (the reference layout; specified
+// in tests/palette_oracle.c and tests/cell_types_oracle.c).  kPaletteAlbedo: the albedo of the final camera-chain hit is its
+// palette entry.  kCellTypes: a hit on a voxel whose colour has type Cell::Mirror reflects on the face it hit (below).  The
+// frame kernels have kPalette with kMirror: mirror_y1 = 0 matches no face, and without kCellTypes the tint stays 1.
 template <bool kMirror = false, bool kPalette = kMirror>
 __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& c, int stage, const LsvoResult& r, const LsvoHit& h,
                                              uint32_t pixel, uint32_t sample, float SCALE, float n_norm, NextRay& nr,
@@ -119,9 +120,25 @@ __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& 
     switch (stage) {
         case kPrimary: {                                                   // raycaster.hpp:131-145
             if (!r.hit) return kDone;
-            if (kMirror) {
-                const int vy = int((h.corner[1] - 1.0f) * float(1 << L.depth));
-                if (c.bounds < L.max_bounds && vy == L.mirror_y1 - 1 && h.normal[1] != 0.0f && h.normal[0] == 0.0f && h.normal[2] == 0.0f) {
+            // A camera-chain hit reflects when bounds < max_bounds and either rule holds: the lake (top faces of layer
+            // mirror_y1 - 1) or, with kCellTypes, a voxel whose colour is Cell::Mirror hit on exactly one face.  Zero normals (a
+            // ray that started inside a solid) and edge or corner hits do not reflect.
+            const bool lake = kMirror && int((h.corner[1] - 1.0f) * float(1 << L.depth)) == L.mirror_y1 - 1 && h.normal[1] != 0.0f &&
+                              h.normal[0] == 0.0f && h.normal[2] == 0.0f;
+            uint32_t colour = 1u;
+            // one descent per hit with cell types; without them only the final hit needs its colour (a lake hit is never final)
+            if (kPalette && ((L.palette & kCellTypes) || ((L.palette & kPaletteAlbedo) && !(lake && c.bounds < L.max_bounds)))) {
+                // castRay voxel v = setCell coordinate S-1-v, taken from the hit cell's corner like the lake test above
+                const float S = float(1 << L.depth);
+                const uint32_t S1 = (1u << L.depth) - 1u;
+                const uint32_t slot = lsvo_leaf_slot(ref_nodes, L.depth, S1 - uint32_t(int((h.corner[0] - 1.0f) * S)),
+                                                     S1 - uint32_t(int((h.corner[1] - 1.0f) * S)), S1 - uint32_t(int((h.corner[2] - 1.0f) * S)));
+                if (slot != kNoLeafSlot) colour = __ldg(ref_nodes + slot).x & 0xffu;
+            }
+            if (kMirror || kPalette) {
+                const int faces = int(h.normal[0] != 0.0f) + int(h.normal[1] != 0.0f) + int(h.normal[2] != 0.0f);
+                const bool typed = kPalette && (L.palette & kCellTypes) && faces == 1 && __ldg(L.tex_top + kCellTypesOffset + colour) == 2;
+                if (c.bounds < L.max_bounds && (lake || typed)) {
                     nr.ox = h.pos[0] + h.normal[0] * SCALE * 0.001f;
                     nr.oy = h.pos[1] + h.normal[1] * SCALE * 0.001f;
                     nr.oz = h.pos[2] + h.normal[2] * SCALE * 0.001f;
@@ -129,7 +146,10 @@ __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& 
                     const float r0 = lattice_dim(L, pixel, sample, 8u + 3u * b, -0.5f, 0.5f);
                     const float r1 = lattice_dim(L, pixel, sample, 9u + 3u * b, -0.5f, 0.5f);
                     const float r2 = lattice_dim(L, pixel, sample, 10u + 3u * b, -0.5f, 0.5f);
-                    nr.dx = nr.dx + L.roughness * r0; nr.dy = -nr.dy + L.roughness * r1; nr.dz = nr.dz + L.roughness * r2;
+                    // the component on the normal's one axis is negated (the lake's normal lies along y)
+                    nr.dx = (h.normal[0] != 0.0f ? -nr.dx : nr.dx) + L.roughness * r0;
+                    nr.dy = (h.normal[1] != 0.0f ? -nr.dy : nr.dy) + L.roughness * r1;
+                    nr.dz = (h.normal[2] != 0.0f ? -nr.dz : nr.dz) + L.roughness * r2;
                     normalize3(nr.dx, nr.dy, nr.dz);
                     nr.coef = 0.0f;
                     c.tint = c.tint * 0.8f;
@@ -139,13 +159,7 @@ __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& 
             }
             c.have_hit = true;
             c.nx = h.normal[0]; c.ny = h.normal[1]; c.nz = h.normal[2];
-            if (kPalette && L.palette) {
-                // castRay voxel v = setCell coordinate S-1-v, taken from the hit cell's corner like the mirror test above
-                const float S = float(1 << L.depth);
-                const uint32_t S1 = (1u << L.depth) - 1u;
-                const uint32_t slot = lsvo_leaf_slot(ref_nodes, L.depth, S1 - uint32_t(int((h.corner[0] - 1.0f) * S)),
-                                                     S1 - uint32_t(int((h.corner[1] - 1.0f) * S)), S1 - uint32_t(int((h.corner[2] - 1.0f) * S)));
-                const uint32_t colour = slot != kNoLeafSlot ? (__ldg(ref_nodes + slot).x & 0xffu) : 1u;
+            if (kPalette && (L.palette & kPaletteAlbedo)) {
                 const uint8_t* entry = L.tex_top + kPaletteOffset + 3u * colour;
                 c.tex_r = __ldg(entry); c.tex_g = __ldg(entry + 1); c.tex_b = __ldg(entry + 2);
             } else {

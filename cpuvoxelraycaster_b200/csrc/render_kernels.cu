@@ -615,7 +615,9 @@ __global__ void __launch_bounds__(128, VRT_K6_MIN_CTAS) render_rounds_kernel(Nod
 // reference's renderRay receives from Camera::getRay (main.cpp:147-149) — and gets the sample's colour back.  One thread per
 // ray, the same sample chain as the frame kernels (sun shadow, GI with the Philox numbers of (pixel, sample)), so a ray
 // that equals the frame kernels' primary ray of (pixel, sample) gives exactly that sample's colour.
-// kPalette: albedo from the scene's palette (L.palette); `nodes` is then the reference layout.
+// kPalette: the colour bits of L.palette (palette albedo, mirror voxels); `nodes` is then the reference layout.  With mirror
+// voxels the chain reflects like the frame kernels' (the lake rule, mirror_y1, is a frame parameter and not read here), and
+// distance and complexity are those of the camera ray.
 template <typename Nodes, bool kGuard, bool kPalette = false>
 __global__ void __launch_bounds__(128, 8) shade_rays_kernel(Nodes nodes, RenderLaunch L, uint64_t n, const vrt_shade_job* __restrict__ jobs,
                                                          vrt_shade_result* __restrict__ out) {
@@ -634,6 +636,7 @@ __global__ void __launch_bounds__(128, 8) shade_rays_kernel(Nodes nodes, RenderL
     c.rnd_z = rnd0.z; c.rnd_w = rnd0.w;
     c.light = 0.f; c.irr0 = 0.f; c.irr1 = 0.f;
     c.have_hit = false; c.gi0_hit = false; c.gi1_hit = false;
+    if (kPalette) { c.tint = 1.0f; c.bounds = 0; }
     NextRay nr;
     nr.ox = job.start[0]; nr.oy = job.start[1]; nr.oz = job.start[2];
     nr.dx = job.direction[0]; nr.dy = job.direction[1]; nr.dz = job.direction[2];
@@ -646,13 +649,13 @@ __global__ void __launch_bounds__(128, 8) shade_rays_kernel(Nodes nodes, RenderL
         LsvoResult r;
         if (stage < kGi0) lsvo_cast_ray2<false, false, kGuard>(nodes, stack, guard, guard_sf, nr.ox, nr.oy, nr.oz, nr.dx, nr.dy, nr.dz, 0.0f, 0.0f, r);
         else lsvo_cast_ray2<true, false, kGuard, true>(nodes, stack, guard, guard_sf, nr.ox, nr.oy, nr.oz, nr.dx, nr.dy, nr.dz, nr.coef, 0.0f, r);
-        if (stage == kPrimary) { complexity = r.complexity; if (r.hit) distance = r.t_min; }   // RayContext, raycaster.hpp:132-133,137
+        if (stage == kPrimary && (!kPalette || c.bounds == 0)) { complexity = r.complexity; if (r.hit) distance = r.t_min; }   // RayContext, raycaster.hpp:132-133,137
         LsvoHit h;
         if (r.hit) lsvo_finish(r, nr.ox, nr.oy, nr.oz, L.depth, h);
         stage = chain_advance<false, kPalette>(L, c, stage, r, h, job.pixel, job.sample, SCALE, n_norm, nr, nodes.slots);
     }
     uint32_t cr = 0, cg = 0, cb = 0;
-    chain_colour(L, c, cr, cg, cb);
+    chain_colour<kPalette>(L, c, cr, cg, cb);
     vrt_shade_result res;
     res.r = uint8_t(cr); res.g = uint8_t(cg); res.b = uint8_t(cb); res.hit = c.have_hit ? 1 : 0;
     res.distance = distance;
@@ -666,7 +669,7 @@ cudaError_t launch_shade_rays(const uint2* nodes, bool compact, const RenderLaun
     if (!n) return cudaSuccess;
     const size_t smem = size_t(L.depth + 1) * 128 * 8;
     const unsigned grid = unsigned((n + 127) / 128);
-    // palette: `nodes` is the reference array whatever the scene's layout (the colours live in its leaf slots)
+    // palette or mirror voxels: `nodes` is the reference array whatever the scene's layout (the colours live in its leaf slots)
     if (L.palette) shade_rays_kernel<RefNodes, true, true><<<grid, 128, smem, stream>>>(RefNodes{nodes}, L, n, d_jobs, d_out);
     else if (compact) shade_rays_kernel<CompactNodes, true><<<grid, 128, smem, stream>>>(CompactNodes{nodes}, L, n, d_jobs, d_out);
     else if (guard_binds(L)) shade_rays_kernel<RefNodes, true><<<grid, 128, smem, stream>>>(RefNodes{nodes}, L, n, d_jobs, d_out);

@@ -308,6 +308,20 @@ class LSVO(Volumetric):
             raise ValueError("the palette must be 256 RGB entries")
         check(lib().vrt_scene_set_palette(self.handle, ptr(p)))
 
+    def set_cell_types(self, types):
+        """types: 256 ints, the Cell::Type of the voxels of each colour (1 = Solid, 2 = Mirror) — camera rays reflect off mirror
+        voxels (vrt_scene_set_cell_types); None = all Solid."""
+        if types is None:
+            check(lib().vrt_scene_set_cell_types(self.handle, None))
+            return
+        t = np.asarray(types).reshape(-1)
+        if t.size != 256:
+            raise ValueError("the cell-type table must have 256 entries")
+        if not np.isin(t, (1, 2)).all():
+            raise ValueError("cell types must be 1 (Solid) or 2 (Mirror)")
+        t = np.ascontiguousarray(t, np.uint8)
+        check(lib().vrt_scene_set_cell_types(self.handle, ptr(t)))
+
     def set_cells(self, xyz, solid=True):
         """Dynamic scene: adds (solid) or removes voxels of a from_voxels(on_device=True) world and re-flattens it on
         the device — what LSVO::setCell would do if it were not a no-op (lsvo.hpp:26)."""

@@ -244,9 +244,9 @@ typedef struct vrt_render_params {
     int32_t checker_area_height; /* height of the reference's thread areas (RENDER_HEIGHT / area_count, main.cpp:132;
                                   * 135 in the demo): area_start(y) = y - y % area_height.  0 = one area (start 0) */
     int32_t mirror_y1;           /* LSVO scenes: 1 + y (castRay voxel coordinates) of the voxel layer whose TOP faces are
-                                  * Cell::Mirror (cell.hpp:8) — the LSVO has one shared cell (lsvo.hpp:21-23), so mirrors are a rule:
-                                  * e.g. the flat valley floors of the demo terrain.  A mirror hit reflects like on grid scenes
-                                  * (roughness, max_bounds, tint 0.8 per bounce; DESIGN.md §2).  0 = no mirrors */
+                                  * Cell::Mirror (cell.hpp:8) — a geometric rule (a lake), e.g. the flat valley floors of the demo
+                                  * terrain; vrt_scene_set_cell_types makes mirrors of painted voxels instead.  A mirror hit reflects
+                                  * like on grid scenes (roughness, max_bounds, tint 0.8 per bounce; DESIGN.md §2).  0 = no lake */
     int32_t autofocus;           /* 1 = LSVO scenes: focal length from the centre ray, cast on the device in front of the
                                   * frame (Camera::getClosestPoint camera_controller.hpp:56-60 + main.cpp:114-121:
                                   * distance * 2^depth, or 100 on a miss); cam->focal_length is ignored.  No host
@@ -269,6 +269,17 @@ int vrt_scene_set_textures(vrt_scene* scene, const uint8_t* top_rgb, const uint8
  * textures, the reference node layout and render_variant 0, 2 or 4 (VRT_ERR_UNSUPPORTED otherwise); vrt_shade_rays and
  * vrt_render_distributed honour it.  rgb = 256*3 bytes (entry c is the albedo of colour c); NULL = back to the textures. */
 int vrt_scene_set_palette(vrt_scene* scene, const uint8_t* rgb);
+/* LSVO scenes: mirror voxels.  types[c] is the Cell::Type (cell.hpp:8) of the voxels of colour c: 1 = Cell::Solid (the default
+ * of every colour), 2 = Cell::Mirror; any other value, 0 included, is VRT_ERR_INVALID.  NULL (or a table without a Mirror
+ * entry) = all Solid.  While a Mirror entry is set, a hit of the camera ray or of a reflected ray on a voxel whose colour is
+ * Mirror reflects when bounds < max_bounds and the raw hit normal has exactly one non-zero component: the ray continues from
+ * hit + normal * 0.001 / 2^depth with that direction component negated, jittered by roughness and re-normalised, tint * 0.8 —
+ * the rule of mirror_y1, which still applies on its own.  Zero normals (a ray that started inside a solid) and edge or corner
+ * hits shade as ordinary hits, and so do sun-shadow and GI rays, which see mirror voxels as solids.  Works with and without a
+ * palette; on a heightfield every voxel has colour 1.  Frames need the reference node layout, render_variant 0, 2 or 4
+ * (VRT_ERR_UNSUPPORTED otherwise) and max_bounds 0..16; vrt_shade_rays and vrt_render_distributed honour the table.
+ * VRT_ERR_UNSUPPORTED for grid and SVO scenes, which have per-cell types of their own. */
+int vrt_scene_set_cell_types(vrt_scene* scene, const uint8_t* types /* 256 */);
 
 /* d_accum: device uint32 [height*width*4] r,g,b,count sums (RayCaster::colors, raycaster.hpp:259; the
  * integer sums equal the reference's double accumulators exactly).  Rows outside [row_begin,row_end)
@@ -296,7 +307,8 @@ int vrt_beam_floors(vrt_scene* scene, const vrt_camera* cam, const vrt_render_pa
  * renderRay (raycaster.hpp:67-92) with the ray Camera::getRay produced (main.cpp:147-149): start and direction in the
  * normalised [1,2]^3 frame.  Returns each ray's ColorResult: the shaded 8-bit colour (texture, sun shadow, GI when
  * p->use_gi, with the Philox numbers of (pixel, sample)), hit flag, HitPoint::distance and complexity of the primary ray.
- * Only the shading fields of *p are read (light_position, use_gi, gi_bounces, seed); LSVO scenes.  This is the
+ * Only the shading fields of *p are read (light_position, use_gi, gi_bounces, seed; roughness and max_bounds with mirror voxels,
+ * vrt_scene_set_cell_types, whose reflections it follows: distance and complexity are then the camera ray's); LSVO scenes.  This is the
  * compatibility path for hosts that keep the reference's loop structure — frames should use vrt_render. */
 typedef struct vrt_shade_job {
     float start[3];

@@ -295,6 +295,13 @@ struct LSVO : public Volumetric {
     // frames take the albedo of colour c from rgb[3c..3c+2] (256 entries) instead of the textures, until clearPalette()
     void setPalette(const uint8_t rgb[768]) { vrt::check(vrt_scene_set_palette(m_scene.s, rgb)); }
     void clearPalette() { vrt::check(vrt_scene_set_palette(m_scene.s, nullptr)); }
+    // voxels of colour c are Cell::Mirror where types[c] is, Cell::Solid (the default) otherwise; until clearCellTypes()
+    void setCellTypes(const Cell::Type (&types)[256]) {
+        uint8_t t[256];
+        for (int c = 0; c < 256; ++c) t[c] = uint8_t(types[c]);
+        vrt::check(vrt_scene_set_cell_types(m_scene.s, t));
+    }
+    void clearCellTypes() { vrt::check(vrt_scene_set_cell_types(m_scene.s, nullptr)); }
 
     std::vector<vrt_lnode> data;                        // LNode[] in the reference layout (lsvo.hpp:287)
     const vrt_lnode* raw_data = nullptr;                // lsvo.hpp:288
@@ -715,7 +722,7 @@ private:
         p.seed_lo = seed_lo; p.seed_hi = seed_hi;
         p.light_position[0] = light_position.x; p.light_position[1] = light_position.y; p.light_position[2] = light_position.z;
         p.use_gi = use_gi; p.gi_bounces = gi_bounces; p.use_samples = use_samples;
-        p.max_bounds = int32_t(max_bounds);
+        p.roughness = roughness; p.max_bounds = int32_t(max_bounds);   // read with mirror voxels (LSVO::setCellTypes)
         return p;
     }
     uint32_t pending_count(uint32_t pixel) {            // samples of this pixel already queued in this batch
