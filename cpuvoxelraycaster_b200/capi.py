@@ -14,7 +14,9 @@ HIT = np.dtype([("position", "f4", 3), ("distance", "f4"), ("normal", "f4", 3), 
                 ("voxel_coord", "f4", 2), ("flags", "u4"), ("scale", "i4"), ("voxel", "i4", 3), ("face", "u4")])
 SHADE_JOB = np.dtype([("start", "f4", 3), ("pixel", "u4"), ("direction", "f4", 3), ("sample", "u4")])
 SHADE_RESULT = np.dtype([("r", "u1"), ("g", "u1"), ("b", "u1"), ("hit", "u1"), ("distance", "f4"), ("complexity", "u4"), ("reserved", "u4")])
+POINT_LIGHT = np.dtype([("position", "f4", 3), ("color", "f4", 3), ("range", "f4"), ("reserved", "u4")])
 assert HIT.itemsize == 64 and LNODE.itemsize == 8 and SHADE_JOB.itemsize == 32 and SHADE_RESULT.itemsize == 16
+assert POINT_LIGHT.itemsize == 32
 
 
 class Camera(C.Structure):
@@ -80,6 +82,7 @@ _SIGNATURES = {
     "vrt_scene_set_textures": (C.c_int, [_vp, _vp, _vp]),
     "vrt_scene_set_palette": (C.c_int, [_vp, _vp]),
     "vrt_scene_set_cell_types": (C.c_int, [_vp, _vp]),
+    "vrt_scene_set_point_lights": (C.c_int, [_vp, _vp, _u32]),
     "vrt_scene_paint_cells": (C.c_int, [_vp, _vp, _vp, _u64, C.POINTER(_u64)]),
     "vrt_scene_cell_colors": (C.c_int, [_vp, _vp, _u64, _vp]),
     "vrt_render_accumulate_device": (C.c_int, [_vp, C.POINTER(Camera), C.POINTER(RenderParams), _vp]),

@@ -793,6 +793,8 @@ int check_render_args(const vrt_scene* sc, const vrt_camera* cam, const vrt_rend
     }
     if (cam && sc->has_palette && (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3))
         return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": palette frames need the reference node layout and render_variant 0, 2 or 4");
+    if (cam && sc->has_lights && (sc->use_compact || sc->ctx->render_variant == 1 || sc->ctx->render_variant == 3))
+        return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": point lights need the reference node layout and render_variant 0, 2 or 4");
     if (cam && p->autofocus && sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": autofocus needs an LSVO scene");
     if (cam && p->checker && sc->kind == VRT_SCENE_LSVO && (sc->ctx->render_variant == 1 || sc->ctx->render_variant >= 3))
         return fail(VRT_ERR_UNSUPPORTED, std::string(who) + ": the checkerboard needs render_variant 0 or 2");
@@ -822,7 +824,8 @@ vrt::RenderLaunch make_launch(const vrt_scene* sc, const vrt_camera* cam, const 
     L.roughness = p->roughness;
     L.max_bounds = p->max_bounds;
     L.mirror_y1 = sc->kind == VRT_SCENE_LSVO ? p->mirror_y1 : 0;
-    L.palette = (sc->has_palette ? vrt::kPaletteAlbedo : 0) | (sc->has_cell_types ? vrt::kCellTypes : 0);
+    L.palette = (sc->has_palette ? vrt::kPaletteAlbedo : 0) | (sc->has_cell_types ? vrt::kCellTypes : 0) |
+                (sc->has_lights ? vrt::kPointLights : 0);
     L.checker = p->checker; L.checker_area_height = p->checker_area_height;
     L.focal = p->autofocus ? reinterpret_cast<const float*>(sc->d_counters + kFocalSlot) : nullptr;
     L.tile_step = p->tile_step > 1 ? p->tile_step : 1;
@@ -878,6 +881,40 @@ int vrt_scene_set_cell_types(vrt_scene* sc, const uint8_t* types) {
     VRT_CUDA(cudaMemcpyAsync(sc->d_tex + vrt::kCellTypesOffset, types, 256, cudaMemcpyHostToDevice, sc->ctx->stream));
     VRT_CUDA(cudaStreamSynchronize(sc->ctx->stream));
     sc->has_cell_types = true;
+    return VRT_OK;
+}
+
+int vrt_scene_set_point_lights(vrt_scene* sc, const vrt_point_light* lights, uint32_t n) {
+    if (!sc) return fail(VRT_ERR_INVALID, "vrt_scene_set_point_lights: scene is NULL");
+    if (sc->kind != VRT_SCENE_LSVO) return fail(VRT_ERR_UNSUPPORTED, "vrt_scene_set_point_lights: needs an LSVO scene");
+    if (n > uint32_t(vrt::kMaxPointLights)) return fail(VRT_ERR_INVALID, "vrt_scene_set_point_lights: at most 16 lights");
+    if (n && !lights) return fail(VRT_ERR_INVALID, "vrt_scene_set_point_lights: lights is NULL");
+    float block[1 + vrt::kMaxPointLights * vrt::kPointLightFloats];
+    const uint32_t count = n;
+    std::memcpy(block, &count, 4);
+    for (uint32_t i = 0; i < n; ++i) {
+        const vrt_point_light& l = lights[i];
+        for (int a = 0; a < 3; ++a) {
+            if (!std::isfinite(l.position[a])) return fail(VRT_ERR_INVALID, "vrt_scene_set_point_lights: positions must be finite");
+            if (!std::isfinite(l.color[a]) || l.color[a] < 0.0f)
+                return fail(VRT_ERR_INVALID, "vrt_scene_set_point_lights: colours must be finite and >= 0");
+        }
+        if (!(l.range > 0.0f)) return fail(VRT_ERR_INVALID, "vrt_scene_set_point_lights: ranges must be > 0 (+inf allowed)");
+        float* r = block + 1 + vrt::kPointLightFloats * i;
+        r[0] = l.position[0]; r[1] = l.position[1]; r[2] = l.position[2];
+        r[3] = l.color[0]; r[4] = l.color[1]; r[5] = l.color[2];
+        r[6] = l.range;
+    }
+    if (!n) {                                                 // no lights: the frames of a scene that never had any
+        sc->has_lights = false;
+        return VRT_OK;
+    }
+    if (int s = use_device(sc->ctx)) return s;
+    if (!sc->d_tex) VRT_CUDA(cudaMalloc(&sc->d_tex, vrt::kTextureBlockBytes));
+    VRT_CUDA(cudaMemcpyAsync(sc->d_tex + vrt::kLightsOffset, block, 4 * (1 + vrt::kPointLightFloats * size_t(n)), cudaMemcpyHostToDevice,
+                             sc->ctx->stream));
+    VRT_CUDA(cudaStreamSynchronize(sc->ctx->stream));
+    sc->has_lights = true;
     return VRT_OK;
 }
 
@@ -978,8 +1015,8 @@ int vrt_shade_rays(vrt_scene* sc, const vrt_render_params* p, uint64_t n, const 
     vrt_render_params q = *p;
     if (q.width <= 0) q.width = 1;
     if (q.height <= 0) q.height = 1;
-    // the palette instance reads colours from the reference array
-    const bool compact = sc->use_compact && !sc->has_palette && !sc->has_cell_types;
+    // the palette instance (palette, cell types, point lights) reads the reference array
+    const bool compact = sc->use_compact && !sc->has_palette && !sc->has_cell_types && !sc->has_lights;
     VRT_CUDA(vrt::launch_shade_rays(compact ? sc->d_compact : sc->d_nodes, compact, make_launch(sc, &cam, &q), n, d_jobs, d_out, ctx->stream));
     ctx->launches += 1;
     VRT_CUDA(cudaMemcpyAsync(out, d_out, size_t(n) * sizeof(vrt_shade_result), cudaMemcpyDeviceToHost, ctx->stream));

@@ -86,10 +86,12 @@ struct vrt_scene {
     // voxel-set scenes once painted: the colour of each resident key (it survives set_cells); an edit gathers the colours of the
     // new key set into the second buffer and swaps the two, so that edits of a painted scene allocate nothing in the steady state
     DeviceBuffer voxel_colors, voxel_colors_next;
-    uint8_t* d_tex = nullptr;                   // kTextureBlockBytes: top (768 B), side (768 B), palette (768 B), cell types (256 B)
+    uint8_t* d_tex = nullptr;                   // kTextureBlockBytes: top (768 B), side (768 B), palette (768 B), cell types (256 B),
+                                                // point lights (count + 16 x 7 floats)
     bool has_tex = false;
     bool has_palette = false;                   // LSVO: frames take the albedo from the palette (vrt_scene_set_palette)
     bool has_cell_types = false;                // LSVO: the cell-type table has a Cell::Mirror entry (vrt_scene_set_cell_types)
+    bool has_lights = false;                    // LSVO: one or more point lights (vrt_scene_set_point_lights)
     DeviceBuffer frame_accum, frame_rgba;       // vrt_render staging
     DeviceBuffer frame_lists;                   // K6: sorted sample lists of the frame in flight
     DeviceBuffer beam_floor;                    // per-tile start distances of the camera rays of the frame in flight

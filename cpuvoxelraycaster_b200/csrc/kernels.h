@@ -79,6 +79,7 @@ struct RenderLaunch {
     // LSVO frames (kMirror kernels) and shade rays, a bit set over the colour of the hit voxel's leaf slot:
     //   kPaletteAlbedo  albedo = palette[colour], the 256 RGB entries at tex_top + kPaletteOffset (else the textures)
     //   kCellTypes      types[colour] == Cell::Mirror reflects camera-chain rays, the 256 bytes at tex_top + kCellTypesOffset
+    //   kPointLights    the point lights at tex_top + kLightsOffset light the final camera-chain hit (their count is in the block)
     // Bits in the alignment gap before `focal` rather than pointers at the end: the struct keeps its 272 bytes, so no kernel
     // parameter behind it moves.
     int palette;
@@ -87,14 +88,18 @@ struct RenderLaunch {
     int checker_area_height;   // thread-area height the checkerboard phase restarts at (0 = never)
 };
 
-constexpr int kPaletteAlbedo = 1, kCellTypes = 2;
+constexpr int kPaletteAlbedo = 1, kCellTypes = 2, kPointLights = 4;
 static_assert(sizeof(RenderLaunch) == 272, "RenderLaunch is a kernel parameter of every frame kernel");
 
-// A scene's texture block on the device: top texture, side texture (16x16 RGB each), the 256-entry RGB palette, then the
-// 256 Cell::Type bytes of the colours (1 = Solid, 2 = Mirror).
+// A scene's texture block on the device: top texture, side texture (16x16 RGB each), the 256-entry RGB palette, the
+// 256 Cell::Type bytes of the colours (1 = Solid, 2 = Mirror), then the point lights: a uint32 count (1..16 while kPointLights
+// is set) and kMaxPointLights records of kPointLightFloats floats {position xyz, colour rgb, range}.
+constexpr int kMaxPointLights = VRT_MAX_POINT_LIGHTS, kPointLightFloats = 7;
 constexpr size_t kPaletteOffset = 1536;
 constexpr size_t kCellTypesOffset = kPaletteOffset + 768;
-constexpr size_t kTextureBlockBytes = kCellTypesOffset + 256;
+constexpr size_t kLightsOffset = kCellTypesOffset + 256;
+constexpr size_t kTextureBlockBytes = kLightsOffset + 4 + kMaxPointLights * kPointLightFloats * 4;
+static_assert(kLightsOffset % 4 == 0, "the lights block is read as uint32 and float");
 
 // main.cpp:143: inside a thread area, rows start at area_start + (x + offset) % 2 and step by 2.
 // Returns the parity x must have for pixel (x, y) to be rendered this frame.

@@ -31,6 +31,10 @@ struct ChainState {
     // mirror reflections (extension, kMirror kernels only): reflections so far, and their accumulated tint
     float tint;
     int bounds;
+    // point lights (extension, kPalette chains only): the light per channel, from the sun term on, and the light whose shadow
+    // ray is in flight (-1: the sun's)
+    float light_r, light_g, light_b;
+    int light_i;
 };
 
 struct NextRay {
@@ -105,6 +109,20 @@ __device__ __forceinline__ float lattice_dim(const RenderLaunch& L, uint32_t pix
     return lattice(word, lo, hi);
 }
 
+// Point light i as seen from the shadow origin o of a hit with raw normal n (DESIGN.md §2, "Point lights"): its distance, the
+// unit vector t to it and dot(t, n).  t is glm::normalize's, and the distance shares its sum of squares.
+__device__ __forceinline__ const float* point_light(const RenderLaunch& L, int i) {
+    return reinterpret_cast<const float*>(L.tex_top + kLightsOffset + 4) + kPointLightFloats * i;
+}
+__device__ __forceinline__ float point_light_view(const float* pl, float ox, float oy, float oz, float nx, float ny, float nz,
+                                                  float& tx, float& ty, float& tz, float& ndotl) {
+    tx = __ldg(pl) - ox; ty = __ldg(pl + 1) - oy; tz = __ldg(pl + 2) - oz;
+    const float dist = sqrtf(dot3(tx, ty, tz, tx, ty, tz));
+    normalize3(tx, ty, tz);
+    ndotl = dot3(tx, ty, tz, nx, ny, nz);
+    return dist;
+}
+
 // The ray of stage `stage` ended with result (r, h).  Returns the next stage and, unless it is kDone, the next ray.
 // kMirror: mirror reflections on LSVO frames (extension specified in oracle/port.c, shade_sample): the top faces of the voxel
 // layer y = L.mirror_y1 - 1 are Cell::Mirror; a mirror hit re-enters kPrimary with the reflected, roughness-jittered ray.
@@ -112,6 +130,8 @@ __device__ __forceinline__ float lattice_dim(const RenderLaunch& L, uint32_t pix
 // in tests/palette_oracle.c and tests/cell_types_oracle.c).  kPaletteAlbedo: the albedo of the final camera-chain hit is its
 // palette entry.  kCellTypes: a hit on a voxel whose colour has type Cell::Mirror reflects on the face it hit (below).  The
 // frame kernels have kPalette with kMirror: mirror_y1 = 0 matches no face, and without kCellTypes the tint stays 1.
+// kPalette also carries the point lights (L.palette & kPointLights, specified in tests/point_lights_oracle.c): after the sun's
+// shadow ray, kShadow hands out one shadow ray per light that passes its cast test, from the sun's origin, before GI starts.
 template <bool kMirror = false, bool kPalette = kMirror>
 __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& c, int stage, const LsvoResult& r, const LsvoHit& h,
                                              uint32_t pixel, uint32_t sample, float SCALE, float n_norm, NextRay& nr,
@@ -176,10 +196,44 @@ __device__ __forceinline__ int chain_advance(const RenderLaunch& L, ChainState& 
             c.tlx = L.light[0] - nr.ox; c.tly = L.light[1] - nr.oy; c.tlz = L.light[2] - nr.oz;   // :152
             normalize3(c.tlx, c.tly, c.tlz);
             nr.dx = c.tlx; nr.dy = c.tly; nr.dz = c.tlz; nr.coef = 0.0f;
+            if (kPalette) c.light_i = -1;
             return kShadow;
         }
         case kShadow: {                                                    // :155-157
-            if (!r.hit) c.light = fmaxf(0.0f, dot3(c.tlx, c.tly, c.tlz, c.nx, c.ny, c.nz));
+            if (kPalette && c.light_i >= 0) {
+                // the shadow ray of point light light_i returned: it still holds the origin and direction of the light's cast
+                // test, from which distance and dot(t, n) are computed again (the same operations, so the same bits).  A hit
+                // beyond the light does not shadow it.
+                const float* pl = point_light(L, c.light_i);
+                float tx, ty, tz, ndotl;
+                const float dist = point_light_view(pl, nr.ox, nr.oy, nr.oz, c.nx, c.ny, c.nz, tx, ty, tz, ndotl);
+                if (!(r.hit && r.t_min < dist)) {
+                    const float w = 1.0f - dist / __ldg(pl + 6);
+                    c.light_r = c.light_r + (__ldg(pl + 3) * ndotl) * w;
+                    c.light_g = c.light_g + (__ldg(pl + 4) * ndotl) * w;
+                    c.light_b = c.light_b + (__ldg(pl + 5) * ndotl) * w;
+                }
+            } else if (kPalette) {                                         // the sun starts the sums (c.light stays unused)
+                c.light_r = r.hit ? 0.0f : fmaxf(0.0f, dot3(c.tlx, c.tly, c.tlz, c.nx, c.ny, c.nz));
+                c.light_g = c.light_r; c.light_b = c.light_r;
+            } else {
+                if (!r.hit) c.light = fmaxf(0.0f, dot3(c.tlx, c.tly, c.tlz, c.nx, c.ny, c.nz));
+            }
+            if (kPalette && (L.palette & kPointLights)) {
+                // the next light in index order that passes the cast test: in range and in front of the face.  A zero normal,
+                // or a light at the origin (NaN), fails it.
+                const int n_lights = int(__ldg(reinterpret_cast<const uint32_t*>(L.tex_top + kLightsOffset)));
+                for (int i = c.light_i + 1; i < n_lights; ++i) {
+                    const float* pl = point_light(L, i);
+                    float tx, ty, tz, ndotl;
+                    const float dist = point_light_view(pl, nr.ox, nr.oy, nr.oz, c.nx, c.ny, c.nz, tx, ty, tz, ndotl);
+                    if (dist < __ldg(pl + 6) && ndotl > 0.0f) {
+                        nr.dx = tx; nr.dy = ty; nr.dz = tz;                // origin and coef 0 stay the sun shadow ray's
+                        c.light_i = i;
+                        return kShadow;
+                    }
+                }
+            }
             if (!L.use_gi) return kDone;
             // getGlobalIllumination, first bounce, :169-194 — from the primary hit
             const float c1 = lattice(c.rnd_z, -1000.0f, 1000.0f), c2 = lattice(c.rnd_w, -1000.0f, 1000.0f);   // :180-181
@@ -237,10 +291,12 @@ __device__ __forceinline__ void chain_colour(const RenderLaunch& L, const ChainS
         if (L.gi_bounces >= 2) irr = irr + (c.gi1_hit ? fminf(0.5f, c.irr1 * c.dot_gi1) : 0.0f);
         gi = fmaxf(0.0f, 1000000.0f * fminf(0.5f, irr * c.dot_gi0) / 1.0f);   // :201,:206
     }
-    const float f = fminf(1.0f, fmaxf(0.0f, c.light + gi));                // :163
-    if (kMirror) {
-        sum_r += mul_u8(mul_u8(c.tex_r, f), c.tint); sum_g += mul_u8(mul_u8(c.tex_g, f), c.tint); sum_b += mul_u8(mul_u8(c.tex_b, f), c.tint);
+    if (kMirror) {                                                         // :163 per channel: the point lights are coloured
+        const float fr = fminf(1.0f, fmaxf(0.0f, c.light_r + gi)), fg = fminf(1.0f, fmaxf(0.0f, c.light_g + gi)),
+                    fb = fminf(1.0f, fmaxf(0.0f, c.light_b + gi));
+        sum_r += mul_u8(mul_u8(c.tex_r, fr), c.tint); sum_g += mul_u8(mul_u8(c.tex_g, fg), c.tint); sum_b += mul_u8(mul_u8(c.tex_b, fb), c.tint);
     } else {
+        const float f = fminf(1.0f, fmaxf(0.0f, c.light + gi));            // :163
         sum_r += mul_u8(c.tex_r, f); sum_g += mul_u8(c.tex_g, f); sum_b += mul_u8(c.tex_b, f);
     }
 }

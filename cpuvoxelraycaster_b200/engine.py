@@ -322,6 +322,30 @@ class LSVO(Volumetric):
         t = np.ascontiguousarray(t, np.uint8)
         check(lib().vrt_scene_set_cell_types(self.handle, ptr(t)))
 
+    def set_point_lights(self, positions, colors=None, ranges=None):
+        """Point lights (vrt_scene_set_point_lights): positions (n,3) in the normalised castRay frame of light_position, colors (n,3)
+        linear RGB >= 0 (1,1,1 = white), ranges (n,) > 0 (inf allowed); n <= 16.  None (or n = 0) clears them."""
+        if positions is None:
+            check(lib().vrt_scene_set_point_lights(self.handle, None, 0))
+            return
+        pos = np.asarray(positions, np.float32)
+        n = len(pos) if pos.ndim == 2 else -1
+        col = np.asarray(colors, np.float32) if colors is not None else None
+        rng = np.asarray(ranges, np.float32) if ranges is not None else None
+        if n < 0 or pos.shape != (n, 3) or col is None or col.shape != (n, 3) or rng is None or rng.shape != (n,):
+            raise ValueError("point lights need positions (n,3), colors (n,3) and ranges (n,)")
+        if n > 16:
+            raise ValueError("at most 16 point lights")
+        if not np.isfinite(pos).all():
+            raise ValueError("light positions must be finite")
+        if not (np.isfinite(col).all() and (col >= 0).all()):
+            raise ValueError("light colours must be finite and >= 0")
+        if not (rng > 0).all():
+            raise ValueError("light ranges must be > 0 (inf allowed)")
+        a = np.zeros(n, capi.POINT_LIGHT)
+        a["position"], a["color"], a["range"] = pos, col, rng
+        check(lib().vrt_scene_set_point_lights(self.handle, ptr(a) if n else None, n))
+
     def set_cells(self, xyz, solid=True):
         """Dynamic scene: adds (solid) or removes voxels of a from_voxels(on_device=True) world and re-flattens it on
         the device — what LSVO::setCell would do if it were not a no-op (lsvo.hpp:26)."""

@@ -280,6 +280,28 @@ int vrt_scene_set_palette(vrt_scene* scene, const uint8_t* rgb);
  * (VRT_ERR_UNSUPPORTED otherwise) and max_bounds 0..16; vrt_shade_rays and vrt_render_distributed honour the table.
  * VRT_ERR_UNSUPPORTED for grid and SVO scenes, which have per-cell types of their own. */
 int vrt_scene_set_cell_types(vrt_scene* scene, const uint8_t* types /* 256 */);
+/* LSVO scenes: point lights (extension, DESIGN.md §2), in the normalised castRay frame of light_position (the cube is [1,2]^3;
+ * setCell voxel v has its centre at 1 + (S-1-v + 0.5)/S on each axis).  color is a linear RGB intensity (1,1,1 = white);
+ * range > 0, +inf allowed. */
+typedef struct vrt_point_light {
+    float position[3];
+    float color[3];
+    float range;
+    uint32_t reserved;
+} vrt_point_light;
+#define VRT_MAX_POINT_LIGHTS 16
+/* Sets the scene's 0..16 point lights (n = 0 clears them).  The final hit of a camera chain (the hit the sun shades: the camera
+ * ray's, or the last one after mirror bounces) with raw normal n and sun shadow origin hp = hit + n * 0.001 / 2^depth is lit,
+ * after the sun, by each light i in index order:
+ *     v = P_i - hp, dist = |v|, t = normalize(v), ndotl = dot(t, n)
+ *     a shadow ray (origin hp, direction t) is cast iff dist < range_i and ndotl > 0 (counted as a shadow ray, class 1);
+ *     unless it hits at a distance < dist:  L_c += (color_i,c * ndotl) * (1 - dist / range_i)
+ * L_c starts at the sun term; the sample's colour is mult(mult(albedo_c, min(1, max(0, L_c + gi))), tint) per channel — with no
+ * lights the frame is unchanged.  A hit beyond the light does not shadow it; GI stays lit by the sun alone.  Frames need the
+ * reference node layout and render_variant 0, 2 or 4 (VRT_ERR_UNSUPPORTED otherwise); vrt_shade_rays and vrt_render_distributed
+ * honour the lights.  VRT_ERR_INVALID: lights == NULL with n > 0, n > 16, a non-finite position, a negative or non-finite colour
+ * component, a range <= 0 or NaN.  VRT_ERR_UNSUPPORTED for grid and SVO scenes.  Uploads on the context stream and waits. */
+int vrt_scene_set_point_lights(vrt_scene* scene, const vrt_point_light* lights, uint32_t n);
 
 /* d_accum: device uint32 [height*width*4] r,g,b,count sums (RayCaster::colors, raycaster.hpp:259; the
  * integer sums equal the reference's double accumulators exactly).  Rows outside [row_begin,row_end)
@@ -308,7 +330,8 @@ int vrt_beam_floors(vrt_scene* scene, const vrt_camera* cam, const vrt_render_pa
  * normalised [1,2]^3 frame.  Returns each ray's ColorResult: the shaded 8-bit colour (texture, sun shadow, GI when
  * p->use_gi, with the Philox numbers of (pixel, sample)), hit flag, HitPoint::distance and complexity of the primary ray.
  * Only the shading fields of *p are read (light_position, use_gi, gi_bounces, seed; roughness and max_bounds with mirror voxels,
- * vrt_scene_set_cell_types, whose reflections it follows: distance and complexity are then the camera ray's); LSVO scenes.  This is the
+ * vrt_scene_set_cell_types, whose reflections it follows: distance and complexity are then the camera ray's; the scene's point
+ * lights, vrt_scene_set_point_lights); LSVO scenes.  This is the
  * compatibility path for hosts that keep the reference's loop structure — frames should use vrt_render. */
 typedef struct vrt_shade_job {
     float start[3];

@@ -302,6 +302,10 @@ struct LSVO : public Volumetric {
         vrt::check(vrt_scene_set_cell_types(m_scene.s, t));
     }
     void clearCellTypes() { vrt::check(vrt_scene_set_cell_types(m_scene.s, nullptr)); }
+    // up to 16 point lights (vrt_scene_set_point_lights) light the frames of every RayCaster of this scene, render() and the
+    // queued renderRay() alike, until clearPointLights()
+    void setPointLights(const vrt_point_light* lights, uint32_t n) { vrt::check(vrt_scene_set_point_lights(m_scene.s, lights, n)); }
+    void clearPointLights() { vrt::check(vrt_scene_set_point_lights(m_scene.s, nullptr, 0)); }
 
     std::vector<vrt_lnode> data;                        // LNode[] in the reference layout (lsvo.hpp:287)
     const vrt_lnode* raw_data = nullptr;                // lsvo.hpp:288
